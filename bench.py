@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — throughput of the EB-CADRL hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[1] — EB-CADRL entity-typed agents + static
@@ -26,6 +26,11 @@ One "step" = what the reference does per env step with the policy in the loop
 `value` is the POLICY-IN-THE-LOOP metric (every agent-step pays a full 81-action lookahead through the value
 network); `sim_only` is SURVEY 8d(i)'s committed-step path, the one north_star's 1e8 agent-steps/s target is
 stated on.  `--workload cfg5` times the training loop instead (rl/train.py semantics, see run_cfg5).
+
+`--dump-outputs DIR` writes what the last of the K timed steps handed back (DUMPED: values and action values of the
+decision, the chosen action, reward / done / event, the state after the step and the re-initialisation) as
+DIR/<name>.npy, so that two builds can be compared output for output: scenes and weights are fixed, so the same
+arguments give the same inputs.
 """
 import argparse
 import json
@@ -51,6 +56,8 @@ EPISODES_PER_GPU = 4096
 N_ACTIONS = 81
 METRIC = "agent_steps_per_sec"
 UNIT = "agent-steps/s"
+DUMPED = ("values", "action_values", "argmax", "reward", "done", "event", "hum_pv", "rob_pv")   # BatchedSim, [N, ...]
+DUMP_BYTES = 64_000_000
 
 
 WORKLOADS = {   # name -> (synth shape, robot kinematics, entity-typed rows, weights fixture, episodes per GPU)
@@ -94,6 +101,24 @@ def value_net_weights(D=17, seed=0, fixture="weights_ebcadrl.npz"):
             sd["%s.%d.weight" % (name, 2 * i)] = rng.uniform(-b, b, (ds[i + 1], ds[i])).astype(np.float32)
             sd["%s.%d.bias" % (name, 2 * i)] = rng.uniform(-b, b, ds[i + 1]).astype(np.float32)
     return sd, "seeded random init"
+
+
+def dump_outputs(path, arrays, budget=DUMP_BYTES):
+    """Write each [N, ...] array of `arrays` as path/<name>.npy, float32 / float64 kept, integers and flags as float64,
+    plus episode_index.npy (the rows written).  Above `budget` bytes in all, every array keeps the same rows: a
+    fixed-seed sample of the episodes, so that two runs of the same arguments write the same files."""
+    out = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    n = len(next(iter(out.values())))
+    room = budget - 256 * (len(out) + 1)                          # .npy headers
+    row_bytes = sum(v.nbytes for v in out.values()) // n + 8      # + its episode_index entry
+    idx = np.arange(n)
+    if n * row_bytes > room:
+        idx = np.sort(np.random.default_rng(0).choice(n, room // row_bytes, replace=False))
+        out = {k: v[idx] for k, v in out.items()}
+    out["episode_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 def flops_per_eval(sd, n):
@@ -384,7 +409,11 @@ def main():
                     help="length of the extra back-to-back region reported under `sustained` (0 = skip)")
     ap.add_argument("--value-mode", default="tc_fp16x2", choices=["fp32", "tc_fp32", "tc_fp16x2", "tc_bf16"],
                     help="K4 arithmetic; tc_fp16x2 (tcgen05, fp32-accurate operand splitting) is the parity mode")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (at most 64 MB; rank 0's episodes)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "cfg5"):
+        ap.error("--dump-outputs covers the --impl b200 step workloads (%s)" % ", ".join(sorted(WORKLOADS)))
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -465,6 +494,8 @@ def main():
     wall1 = time.time()
     launches = sim.launch_count() - launches0
     elapsed_ms = t_begin.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: getattr(sim, k).cpu().numpy() for k in DUMPED})
     phase_names = ["orca", "lookahead", "value", "select", "step", "reset"]
     phase_ms = dict.fromkeys(phase_names, 0.0)
     for s in range(args.steps):

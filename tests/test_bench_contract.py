@@ -1,6 +1,7 @@
 """bench.py's bookkeeping, checked on the CPU: the roofline numerator is SURVEY 8d's algorithmic FLOP count, the
-workloads are BASELINE.json's configurations, and the reference arm prints the contract's keys (it runs the oracle
-port on the host cores; no GPU involved)."""
+workloads are BASELINE.json's configurations, the reference arm prints the contract's keys (it runs the oracle
+port on the host cores; no GPU involved) and --dump-outputs keeps to its budget; on the GPU, --dump-outputs end to
+end."""
 import importlib.util
 import json
 import os
@@ -8,6 +9,7 @@ import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -57,3 +59,55 @@ def test_reference_arm_prints_the_contract_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
                          capture_output=True, text=True, timeout=120, env=dict(os.environ, RANK="1", WORLD_SIZE="2"))
     assert out.returncode == 0 and not [l for l in out.stdout.splitlines() if l.startswith("{")]
+
+
+def test_dump_outputs_keeps_the_same_rows_within_the_budget(tmp_path):
+    b = _bench()
+    rng = np.random.default_rng(1)
+    n = 1000
+    arrays = {"values": rng.random((n, 81), dtype=np.float32), "reward": rng.random(n),
+              "argmax": rng.integers(0, 81, n, dtype=np.int32), "done": (rng.random(n) < 0.1).astype(np.uint8)}
+
+    def written(d):
+        return {f[:-4]: np.load(os.path.join(d, f)) for f in os.listdir(d)}
+
+    b.dump_outputs(str(tmp_path / "whole"), arrays)
+    whole = written(str(tmp_path / "whole"))
+    assert set(whole) == set(arrays) | {"episode_index"}
+    assert all(v.dtype in (np.float32, np.float64) for v in whole.values())
+    assert np.array_equal(whole["episode_index"], np.arange(n))
+    for k, v in arrays.items():
+        assert np.array_equal(whole[k], v) and whole[k].dtype == (v.dtype if k in ("values", "reward") else np.float64)
+
+    budget = 100_000
+    for name in ("a", "b"):
+        b.dump_outputs(str(tmp_path / name), arrays, budget=budget)
+    a, a2 = written(str(tmp_path / "a")), written(str(tmp_path / "b"))
+    assert sum(os.path.getsize(str(tmp_path / "a" / f)) for f in os.listdir(str(tmp_path / "a"))) <= budget
+    idx = a["episode_index"].astype(np.int64)
+    assert 0 < len(idx) < n and np.all(np.diff(idx) > 0)
+    for k, v in arrays.items():
+        assert np.array_equal(a[k], v[idx]) and np.array_equal(a[k], a2[k])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_and_follow_steps(tmp_path):
+    """The same arguments dump the same outputs bit for bit; one more timed step dumps a later state."""
+    b = _bench()
+
+    def run(steps, name):
+        d = str(tmp_path / name)
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--episodes", "512", "--steps", str(steps),
+                              "--warmup", "3", "--no-cpu-baseline", "--sustained-seconds", "0", "--dump-outputs", d],
+                             capture_output=True, text=True, timeout=600, env=dict(os.environ, RANK="0", WORLD_SIZE="1"))
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])["steps"] == steps
+        return {f[:-4]: np.load(os.path.join(d, f)) for f in os.listdir(d)}
+
+    first, again, later = run(2, "first"), run(2, "again"), run(3, "later")
+    assert set(first) == set(b.DUMPED) | {"episode_index"}
+    assert first["values"].shape == (512, 81) and np.array_equal(first["episode_index"], np.arange(512))
+    for k, v in first.items():
+        assert v.dtype in (np.float32, np.float64) and np.isfinite(v).all(), k
+        assert np.array_equal(v, again[k]), k
+    assert not np.array_equal(first["hum_pv"], later["hum_pv"])
