@@ -3,8 +3,8 @@
 //   K1 orca_kernel        warp per human: RVO2 neighbour selection + ORCA half-planes + the
 //                         incremental 2-D linear program, lines distributed one per lane
 //                         (simulator/policy/orca.py:85-157 -> rvo2 doStep; SURVEY Appendix A)
-//   K3 lookahead_kernel   warp per (episode, action): swept-disc collisions, occupancy-grid
-//                         test, reward/done/event, next states, rotated joint-state rows
+//   K3 lookahead_kernel   a group of 8, 16 or 32 lanes per (episode, action): swept-disc collisions,
+//                         occupancy-grid test, reward/done/event, next states, rotated joint-state rows
 //                         (simulator/env.py:207-209,388-466; rl/policy/cadrl.py:118-165,236-337)
 //   K5 select_kernel      warp per episode: reward + gamma^(dt v_pref) V, first-max argmax
 //                         (rl/policy/multi_human_rl.py:72-82)
@@ -32,25 +32,14 @@ struct Line { float px, py, dx, dy; };
 __device__ __forceinline__ float det2(float ax, float ay, float bx, float by) { return ax * by - ay * bx; }
 __device__ __forceinline__ float dot2(float ax, float ay, float bx, float by) { return ax * bx + ay * by; }
 
-__device__ __forceinline__ double warp_min_d(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(FULL, v, o));
-  return v;
-}
-
-// The group's ORCA lines: line index = lane + GW * chunk.  A group = the GW lanes that solve one agent's LP: the whole
-// warp (GW = 32), or a half warp (GW = 16: two agents per warp, every shuffle / ballot / reduction confined to the
-// half through its member mask `m`; `lane` is then the lane index inside the half).  LPL (lines per lane) = 1 on the
-// reference's live path (at most max_neighbors agent lines), 2 when obstacle half-planes are enabled (up to 64
-// lines, obstacle lines first; GW = 32 only).  Every function below is the same arithmetic for all (GW, LPL).
-template <int LPL> struct Lines { Line l[LPL]; };
-
+// Lane groups: a group = GW consecutive lanes of a warp (GW = 8, 16 or 32), its first lane `lane & (32 - GW)`.  Every
+// ballot / shuffle / reduction below is confined to the group; `m` is the member mask of the lanes taking part (K1: the
+// group's own lanes, group_mask; K3: FULL, its groups are the convergent lanes of whole warps).
 template <int GW> __device__ __forceinline__ unsigned group_mask() {
-  return GW == 32 ? FULL : (0xFFFFu << ((threadIdx.x & 31) & 16));
+  return (FULL >> (32 - GW)) << ((threadIdx.x & 31) & (32 - GW));
 }
 template <int GW> __device__ __forceinline__ unsigned grp_ballot(unsigned m, bool p) {
-  const unsigned b = __ballot_sync(m, p);
-  return GW == 32 ? b : ((b >> ((threadIdx.x & 31) & 16)) & 0xFFFFu);
+  return (__ballot_sync(m, p) >> ((threadIdx.x & 31) & (32 - GW))) & (FULL >> (32 - GW));
 }
 template <int GW> __device__ __forceinline__ float grp_min_f(unsigned m, float v) {
 #pragma unroll
@@ -62,6 +51,18 @@ template <int GW> __device__ __forceinline__ float grp_max_f(unsigned m, float v
   for (int o = GW / 2; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(m, v, o, GW));
   return v;
 }
+template <int GW> __device__ __forceinline__ double grp_min_d(unsigned m, double v) {
+#pragma unroll
+  for (int o = GW / 2; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(m, v, o, GW));
+  return v;
+}
+
+// The group's ORCA lines: line index = lane + GW * chunk.  A group = the GW lanes that solve one agent's LP: the whole
+// warp (GW = 32), or a half warp (GW = 16: two agents per warp, every shuffle / ballot / reduction confined to the
+// half through its member mask `m`; `lane` is then the lane index inside the half).  LPL (lines per lane) = 1 on the
+// reference's live path (at most max_neighbors agent lines), 2 when obstacle half-planes are enabled (up to 64
+// lines, obstacle lines first; GW = 32 only).  Every function below is the same arithmetic for all (GW, LPL).
+template <int LPL> struct Lines { Line l[LPL]; };
 
 template <int LPL, int GW>
 __device__ __forceinline__ void bcast_line(unsigned m, const Lines<LPL> &L, int i, float &px, float &py, float &dx,
@@ -799,29 +800,13 @@ struct Outcome {
   int done, event;
 };
 
-// The humans of one episode, two per lane.
+// The humans of one episode over a group of G lanes: lane l holds humans l + G * chunk, a second chunk only for G = 32
+// (K3 gives a smaller group only states of at most G rows).
 struct EpisodeHumans {
   float4 pv[2];
   float rad[2];
   int type[2];   // -1 = empty slot
 };
-
-__device__ __forceinline__ void load_humans(const ebc_config &c, const ebc_state &st, int e, int H, int lane,
-                                            EpisodeHumans &hm) {
-  const int Hm = c.max_humans;
-#pragma unroll
-  for (int ch = 0; ch < 2; ++ch) {
-    const int h = lane + 32 * ch;
-    hm.type[ch] = -1;
-    hm.pv[ch] = make_float4(0.f, 0.f, 0.f, 0.f);
-    hm.rad[ch] = 0.f;
-    if (h < H) {
-      hm.pv[ch] = reinterpret_cast<const float4 *>(st.hum_pv)[(size_t)e * Hm + h];
-      hm.rad[ch] = st.hum_gr[((size_t)e * Hm + h) * 4 + 3];
-      hm.type[ch] = st.hum_type[(size_t)e * Hm + h];
-    }
-  }
-}
 
 // reward.py:80-181 and the Info classes: the priority chain from the three dmin / four collision flags
 __device__ __forceinline__ void classify_outcome(const ebc_config &c, const float4 rg, double gt, double a1,
@@ -870,10 +855,13 @@ __device__ __forceinline__ void classify_outcome(const ebc_config &c, const floa
   o.reward = reward; o.done = done; o.event = ev;
 }
 
-// env.py:424-444 for one (episode, action), cooperatively by one warp; result warp-uniform.
-__device__ void evaluate_action_warp(const ebc_config &c, const ebc_state &st, int e, int lane,
-                                     const EpisodeHumans &hm, const float4 rp, const float4 rg, double theta,
-                                     double gt, double a0, double a1, Outcome &o) {
+// env.py:424-444 for one (episode, action) of an episode with H humans, cooperatively by a group of G lanes (lane = the
+// index inside it), which load the humans into `hm` (the commit integrates them afterwards); the result is uniform over
+// the group.  The group's lanes take part in full warps (member mask FULL).
+template <int G>
+__device__ void evaluate_action(const ebc_config &c, const ebc_state &st, int e, int lane, int H, const float4 rp,
+                                const float4 rg, double theta, double gt, double a0, double a1, EpisodeHumans &hm,
+                                Outcome &o) {
   const double rpx = rp.x, rpy = rp.y, rrad = rg.w;
   const double dt = c.time_step;
   double avx, avy;
@@ -893,10 +881,23 @@ __device__ void evaluate_action_warp(const ebc_config &c, const ebc_state &st, i
     o.end_x = rpx + o.cs * a0 * dt;
     o.end_y = rpy + o.sn * a0 * dt;
   }
+  const int Hm = c.max_humans;
+#pragma unroll
+  for (int ch = 0; ch < 2; ++ch) {
+    const int h = lane + G * ch;
+    hm.type[ch] = -1;
+    hm.pv[ch] = make_float4(0.f, 0.f, 0.f, 0.f);
+    hm.rad[ch] = 0.f;
+    if ((G == 32 || ch == 0) && h < H) {
+      hm.pv[ch] = reinterpret_cast<const float4 *>(st.hum_pv)[(size_t)e * Hm + h];
+      hm.rad[ch] = st.hum_gr[((size_t)e * Hm + h) * 4 + 3];
+      hm.type[ch] = st.hum_type[(size_t)e * Hm + h];
+    }
+  }
   // env.py:303-338: per type, list order, dmin frozen at the first collision
   double closest[2] = {INFINITY, INFINITY};
   unsigned long long collm = 0ull, typem[3] = {0ull, 0ull, 0ull};
-  const int n_ch = c.max_humans > 32 ? 2 : 1;      // lanes hold humans 32..63 only when the batch has that many
+  const int n_ch = G == 32 && c.max_humans > 32 ? 2 : 1;   // lanes hold humans 32..63 only when the batch has that many
 #pragma unroll
   for (int ch = 0; ch < 2; ++ch) {
     if (ch >= n_ch) break;
@@ -905,22 +906,23 @@ __device__ void evaluate_action_warp(const ebc_config &c, const ebc_state &st, i
     const double vx = (double)hm.pv[ch].z - avx, vy = (double)hm.pv[ch].w - avy;
     const double ex = px + vx * dt, ey = py + vy * dt;
     closest[ch] = point_to_segment_dist0(px, py, ex, ey) - (double)hm.rad[ch] - rrad;
-    collm |= (unsigned long long)__ballot_sync(FULL, valid && closest[ch] < 0.0) << (32 * ch);
+    collm |= (unsigned long long)grp_ballot<G>(FULL, valid && closest[ch] < 0.0) << (G * ch);
 #pragma unroll
     for (int t = 0; t < 3; ++t)
-      typem[t] |= (unsigned long long)__ballot_sync(FULL, valid && hm.type[ch] == t) << (32 * ch);
+      typem[t] |= (unsigned long long)grp_ballot<G>(FULL, valid && hm.type[ch] == t) << (G * ch);
   }
   bool coll[3];
 #pragma unroll
   for (int t = 0; t < 3; ++t) {
     const unsigned long long cm = collm & typem[t];
     coll[t] = cm != 0ull;
-    const int first = coll[t] ? (__ffsll((long long)cm) - 1) : 64;
+    const unsigned lo = (unsigned)cm, hi = (unsigned)(cm >> 32);   // __ffsll(cm) - 1 by halves: fewer registers
+    const int first = lo ? __ffs(lo) - 1 : (hi ? 31 + __ffs(hi) : 64);
     double local = INFINITY;
 #pragma unroll
     for (int ch = 0; ch < 2; ++ch)
-      if (hm.type[ch] == t && lane + 32 * ch < first) local = fmin(local, closest[ch]);
-    o.dmin[t] = warp_min_d(local);
+      if (hm.type[ch] == t && lane + G * ch < first) local = fmin(local, closest[ch]);
+    o.dmin[t] = grp_min_d<G>(FULL, local);
   }
   // env.py:227-261 on the rectangle list
   bool coll_obst = false;
@@ -928,96 +930,19 @@ __device__ void evaluate_action_warp(const ebc_config &c, const ebc_state &st, i
     const int ix = (int)rint((o.end_x + c.map_size_m / 2.0) / c.map_resolution);
     const int iy = (int)rint((o.end_y + c.map_size_m / 2.0) / c.map_resolution);
     const int sz = (int)ceil(rrad / sqrt(2.0) / c.map_resolution);
-    const int G = (int)rint(c.map_size_m / c.map_resolution);
+    const int GR = (int)rint(c.map_size_m / c.map_resolution);
     int sx = ix - sz, ex = sx + sz * 2, sy = iy - sz, ey = sy + sz * 2;
-    sx = max(sx, 0); ex = min(ex, G); sy = max(sy, 0); ey = min(ey, G);
+    sx = max(sx, 0); ex = min(ex, GR); sy = max(sy, 0); ey = min(ey, GR);
     const int R = st.rect_count[e];
     bool hit = false;
     if (ex > sx && ey > sy) {
       const short4 *rc = reinterpret_cast<const short4 *>(st.rect) + (size_t)e * c.max_rects;
-      for (int j = lane; j < R; j += 32) {
+      for (int j = lane; j < R; j += G) {
         const short4 r = rc[j];
         hit |= (sx < r.z && r.x < ex && sy < r.w && r.y < ey);
       }
     }
-    coll_obst = __any_sync(FULL, hit);
-  }
-  classify_outcome(c, rg, gt, a1, coll, coll_obst, o);
-}
-
-// K3 with several (episode, action) pairs per warp: a group of G lanes (8 or 16) does what the warp does in
-// evaluate_action_warp when the episode has at most G humans.  Same arithmetic in the same order; ballots and
-// reductions are confined to the group.
-template <int G>
-__device__ __forceinline__ unsigned group_ballot(bool pred, int sub) {
-  return (__ballot_sync(FULL, pred) >> (sub * G)) & ((1u << G) - 1u);
-}
-template <int G>
-__device__ void evaluate_action_group(const ebc_config &c, const ebc_state &st, int e, int l, int sub, int H,
-                                      const float4 rp, const float4 rg, double theta, double gt, double a0, double a1,
-                                      Outcome &o) {
-  const double rpx = rp.x, rpy = rp.y, rrad = rg.w;
-  const double dt = c.time_step;
-  double avx, avy;
-  if (c.robot_kinematics == EBC_KIN_HOLONOMIC) {
-    avx = a0;
-    avy = a1;
-    o.cs = 0.0; o.sn = 0.0;
-    o.end_x = rpx + a0 * dt;
-    o.end_y = rpy + a1 * dt;
-  } else {
-    const double th = theta + a1;
-    o.cs = cos(th);
-    o.sn = sin(th);
-    avx = a0 * o.cs;
-    avy = a0 * o.sn;
-    o.end_x = rpx + o.cs * a0 * dt;
-    o.end_y = rpy + o.sn * a0 * dt;
-  }
-  float4 pv = make_float4(0.f, 0.f, 0.f, 0.f);
-  float rad = 0.f;
-  int type = -1;
-  if (l < H) {
-    const size_t i = (size_t)e * c.max_humans + l;
-    pv = reinterpret_cast<const float4 *>(st.hum_pv)[i];
-    rad = st.hum_gr[i * 4 + 3];
-    type = st.hum_type[i];
-  }
-  const bool valid = type >= 0 && type <= 2;
-  const double px = (double)pv.x - rpx, py = (double)pv.y - rpy;
-  const double vx = (double)pv.z - avx, vy = (double)pv.w - avy;
-  const double ex = px + vx * dt, ey = py + vy * dt;
-  const double closest = point_to_segment_dist0(px, py, ex, ey) - (double)rad - rrad;
-  const unsigned collm = group_ballot<G>(valid && closest < 0.0, sub);
-  bool coll[3];
-#pragma unroll
-  for (int t = 0; t < 3; ++t) {
-    const unsigned cm = collm & group_ballot<G>(valid && type == t, sub);
-    coll[t] = cm != 0u;
-    const int first = coll[t] ? (__ffs((int)cm) - 1) : 64;
-    double local = (type == t && l < first) ? closest : INFINITY;
-#pragma unroll
-    for (int off = G / 2; off > 0; off >>= 1) local = fmin(local, __shfl_xor_sync(FULL, local, off));
-    o.dmin[t] = local;
-  }
-  bool coll_obst = false;
-  {
-    const int ix = (int)rint((o.end_x + c.map_size_m / 2.0) / c.map_resolution);
-    const int iy = (int)rint((o.end_y + c.map_size_m / 2.0) / c.map_resolution);
-    const int sz = (int)ceil(rrad / sqrt(2.0) / c.map_resolution);
-    const int GR = (int)rint(c.map_size_m / c.map_resolution);
-    int sx = ix - sz, exx = sx + sz * 2, sy = iy - sz, eyy = sy + sz * 2;
-    sx = max(sx, 0); exx = min(exx, GR); sy = max(sy, 0); eyy = min(eyy, GR);
-    const int R = st.rect_count[e];
-    bool hit = false;
-    if (exx > sx && eyy > sy) {
-      const short4 *rc = reinterpret_cast<const short4 *>(st.rect) + (size_t)e * c.max_rects;
-      for (int j = l; j < R; j += G) {
-        const short4 r = rc[j];
-        hit |= (sx < r.z && r.x < exx && sy < r.w && r.y < eyy);
-      }
-    }
-    coll_obst = group_ballot<G>(hit, sub) != 0u;
+    coll_obst = grp_ballot<G>(FULL, hit) != 0u;
   }
   classify_outcome(c, rg, gt, a1, coll, coll_obst, o);
 }
@@ -1063,15 +988,41 @@ __device__ __forceinline__ void store_robot_record(const RobotRow &r, int rotate
   rec[2] = make_float4(cr, sr, 0.0f, 0.0f);
 }
 
-// Build the n x D rows of one state into `tile` (this warp's shared-memory staging area), then
-// stream them out with coalesced stores.  next_state: humans advanced by their ORCA action
-// (agent.py:80-93) when true, current state (multi_human_rl.py:128-149) when false.
-__device__ void build_rows_warp(const ebc_config &c, const ebc_state &st, int e, int lane, int H, int S,
-                                const RobotRow &rr, bool next_state, float *tile, float *dst) {
+// rl/policy/cadrl.py:118-165 propagate(robot) in fp64, narrowed like torch.Tensor([...])
+__device__ __forceinline__ RobotRow propagate_robot(const ebc_config &c, const float4 rp, const float4 rg, double theta,
+                                                    double a0, double a1, const Outcome &o) {
+  RobotRow rr;
+  const double dt = c.time_step;
+  if (c.robot_kinematics == EBC_KIN_HOLONOMIC) {
+    rr.px = (float)((double)rp.x + a0 * dt);
+    rr.py = (float)((double)rp.y + a1 * dt);
+    rr.vx = (float)a0;
+    rr.vy = (float)a1;
+    rr.theta = (float)theta;
+  } else {
+    const double nth = theta + a1;
+    const double nvx = a0 * o.cs, nvy = a0 * o.sn;   // cos / sin of theta + a1, already computed for the collision test
+    rr.px = (float)((double)rp.x + nvx * dt);
+    rr.py = (float)((double)rp.y + nvy * dt);
+    rr.vx = (float)nvx;
+    rr.vy = (float)nvy;
+    rr.theta = (float)nth;
+  }
+  rr.radius = rg.w; rr.gx = rg.x; rr.gy = rg.y; rr.v_pref = rg.z;
+  return rr;
+}
+
+// Build the n x D rows of one state into `tile` (this group's shared-memory staging area; lane l of the group builds
+// rows l, l + G, ...), then stream them out with coalesced stores (dst == NULL: an idle group, nothing to store).
+// next_state: humans advanced by their ORCA action (agent.py:80-93) when true, current state (multi_human_rl.py:128-149)
+// when false.  Every lane of the warp takes part (__syncwarp).
+template <int G>
+__device__ void build_rows(const ebc_config &c, const ebc_state &st, int e, int lane, int H, int S,
+                           const RobotRow &rr, bool next_state, float *tile, float *dst) {
   const int Hm = c.max_humans, Sm = c.max_statics, n = Hm + Sm;
   const int D = c.with_agent_type ? 17 : 13;
   const double dt = c.time_step;
-  for (int r = lane; r < n; r += 32) {
+  for (int r = lane; r < n; r += G) {
     float *row = tile + r * D;
     if (r < H) {
       const float4 p = reinterpret_cast<const float4 *>(st.hum_pv)[(size_t)e * Hm + r];
@@ -1093,67 +1044,17 @@ __device__ void build_rows_warp(const ebc_config &c, const ebc_state &st, int e,
     }
   }
   __syncwarp();
+  if (!dst) return;
   const int total = n * D;
-  for (int i = lane; i < total; i += 32) dst[i] = tile[i];
-  __syncwarp();
+  for (int i = lane; i < total; i += G) dst[i] = tile[i];
 }
 
-// K3
-__global__ void __launch_bounds__(EBC_THREADS)
+// K3, a group of G lanes per (episode, action): G = 8 / 16 for states of at most G rows (32 / G pairs per warp), else
+// the whole warp.  G < 32 keeps four blocks per SM (64 registers).
+template <int G>
+__global__ void __launch_bounds__(EBC_THREADS, G < 32 ? 4 : 0)
 lookahead_kernel(const ebc_config c, const ebc_state st, const double *__restrict__ actions, float *vin,
                  double *reward, uint8_t *done, uint8_t *event, float4 *rec) {
-  extern __shared__ float tiles[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int A = c.n_actions;
-  const long long w = (long long)blockIdx.x * EBC_WARPS_PER_BLOCK + warp;
-  const int e = (int)(w / A), a = (int)(w % A);
-  if (e >= c.n_episodes) return;
-  const int n = c.max_humans + c.max_statics, D = c.with_agent_type ? 17 : 13;
-  const int H = st.hum_count[e], S = st.stat_count[e];
-  EpisodeHumans hm;
-  load_humans(c, st, e, H, lane, hm);
-  const float4 rp = reinterpret_cast<const float4 *>(st.rob_pv)[e];
-  const float4 rg = reinterpret_cast<const float4 *>(st.rob_gr)[e];
-  const double theta = (double)st.rob_theta[e];
-  const double a0 = actions[a * 2], a1 = actions[a * 2 + 1];
-  Outcome o;
-  evaluate_action_warp(c, st, e, lane, hm, rp, rg, theta, st.time[e], a0, a1, o);
-  const size_t ea = (size_t)e * A + a;
-  if (lane == 0) {
-    if (reward) reward[ea] = o.reward;
-    if (done) done[ea] = (uint8_t)o.done;
-    if (event) event[ea] = (uint8_t)o.event;
-  }
-  if (!vin && !rec) return;
-  // rl/policy/cadrl.py:118-165 propagate(robot) in fp64, narrowed like torch.Tensor([...])
-  RobotRow rr;
-  const double dt = c.time_step;
-  if (c.robot_kinematics == EBC_KIN_HOLONOMIC) {
-    rr.px = (float)((double)rp.x + a0 * dt);
-    rr.py = (float)((double)rp.y + a1 * dt);
-    rr.vx = (float)a0;
-    rr.vy = (float)a1;
-    rr.theta = (float)theta;
-  } else {
-    const double nth = theta + a1;
-    const double nvx = a0 * o.cs, nvy = a0 * o.sn;   // cos / sin of theta + a1, already computed for the collision test
-    rr.px = (float)((double)rp.x + nvx * dt);
-    rr.py = (float)((double)rp.y + nvy * dt);
-    rr.vx = (float)nvx;
-    rr.vy = (float)nvy;
-    rr.theta = (float)nth;
-  }
-  rr.radius = rg.w; rr.gx = rg.x; rr.gy = rg.y; rr.v_pref = rg.z;
-  if (rec && lane == 0) store_robot_record(rr, c.rotate_theta, rec + ea * 3);
-  if (vin) build_rows_warp(c, st, e, lane, H, S, rr, true, tiles + (size_t)warp * n * D, vin + ea * (size_t)n * D);
-}
-
-// K3 for episodes with at most G rows per state (G = 8 or 16): 32 / G (episode, action) pairs per warp, lane l of
-// a group holds human l for the outcome and row l for the rotated joint state.  Bit-identical to lookahead_kernel.
-template <int G>
-__global__ void __launch_bounds__(EBC_THREADS)
-lookahead_group_kernel(const ebc_config c, const ebc_state st, const double *__restrict__ actions, float *vin,
-                       double *reward, uint8_t *done, uint8_t *event, float4 *rec) {
   extern __shared__ float tiles[];
   constexpr int GPW = 32 / G;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, sub = lane / G, l = lane % G;
@@ -1171,8 +1072,9 @@ lookahead_group_kernel(const ebc_config c, const ebc_state st, const double *__r
   const float4 rg = reinterpret_cast<const float4 *>(st.rob_gr)[e];
   const double theta = (double)st.rob_theta[e];
   const double a0 = actions[a * 2], a1 = actions[a * 2 + 1];
+  EpisodeHumans hm;
   Outcome o;
-  evaluate_action_group<G>(c, st, e, l, sub, H, rp, rg, theta, st.time[e], a0, a1, o);
+  evaluate_action<G>(c, st, e, l, H, rp, rg, theta, st.time[e], a0, a1, hm, o);
   const size_t ea = (size_t)e * A + a;
   if (live && l == 0) {
     if (reward) reward[ea] = o.reward;
@@ -1180,52 +1082,11 @@ lookahead_group_kernel(const ebc_config c, const ebc_state st, const double *__r
     if (event) event[ea] = (uint8_t)o.event;
   }
   if (!vin && !rec) return;
-  RobotRow rr;
-  const double dt = c.time_step;
-  if (c.robot_kinematics == EBC_KIN_HOLONOMIC) {
-    rr.px = (float)((double)rp.x + a0 * dt);
-    rr.py = (float)((double)rp.y + a1 * dt);
-    rr.vx = (float)a0;
-    rr.vy = (float)a1;
-    rr.theta = (float)theta;
-  } else {
-    const double nth = theta + a1;
-    const double nvx = a0 * o.cs, nvy = a0 * o.sn;
-    rr.px = (float)((double)rp.x + nvx * dt);
-    rr.py = (float)((double)rp.y + nvy * dt);
-    rr.vx = (float)nvx;
-    rr.vy = (float)nvy;
-    rr.theta = (float)nth;
-  }
-  rr.radius = rg.w; rr.gx = rg.x; rr.gy = rg.y; rr.v_pref = rg.z;
+  const RobotRow rr = propagate_robot(c, rp, rg, theta, a0, a1, o);
   if (rec && live && l == 0) store_robot_record(rr, c.rotate_theta, rec + ea * 3);
-  if (!vin) return;               // (warp-uniform: a kernel argument)
-  // rows (n <= G): lane l builds row l in the group's tile, then the group copies it out contiguously
-  float *tile = tiles + (size_t)(warp * GPW + sub) * n * D;
-  if (l < n) {
-    float *row = tile + l * D;
-    const int Hm = c.max_humans, Sm = c.max_statics;
-    if (l < H) {
-      const float4 p = reinterpret_cast<const float4 *>(st.hum_pv)[(size_t)e * Hm + l];
-      const float rad = st.hum_gr[((size_t)e * Hm + l) * 4 + 3];
-      const int ty = st.hum_type[(size_t)e * Hm + l];
-      const float2 nv = reinterpret_cast<const float2 *>(st.hum_nv)[(size_t)e * Hm + l];
-      const float npx = (float)((double)p.x + (double)nv.x * dt);
-      const float npy = (float)((double)p.y + (double)nv.y * dt);
-      rotate_row(rr, npx, npy, nv.x, nv.y, rad, ty, c.rotate_theta, D, row);
-    } else if (l < H + S) {
-      const float4 p = reinterpret_cast<const float4 *>(st.stat)[(size_t)e * Sm + (l - H)];
-      rotate_row(rr, p.x, p.y, 0.0f, 0.0f, p.z, EBC_ADULT_STATIC, c.rotate_theta, D, row);
-    } else {
-      for (int k = 0; k < D; ++k) row[k] = 0.0f;
-    }
-  }
-  __syncwarp();
-  if (live) {
-    float *dst = vin + ea * (size_t)n * D;
-    const int cnt = n * D;
-    for (int i = l; i < cnt; i += G) dst[i] = tile[i];
-  }
+  if (vin)                        // (warp-uniform: a kernel argument)
+    build_rows<G>(c, st, e, l, H, S, rr, true, tiles + (size_t)(warp * GPW + sub) * n * D,
+                  live ? vin + ea * (size_t)n * D : nullptr);
 }
 
 // rl/policy/multi_human_rl.py:128-149
@@ -1240,8 +1101,8 @@ __global__ void __launch_bounds__(EBC_THREADS) transform_kernel(const ebc_config
   RobotRow rr;
   rr.px = rp.x; rr.py = rp.y; rr.vx = rp.z; rr.vy = rp.w;
   rr.radius = rg.w; rr.gx = rg.x; rr.gy = rg.y; rr.v_pref = rg.z; rr.theta = st.rob_theta[e];
-  build_rows_warp(c, st, e, lane, st.hum_count[e], st.stat_count[e], rr, false, tiles + (size_t)warp * n * D,
-                  out + (size_t)e * n * D);
+  build_rows<32>(c, st, e, lane, st.hum_count[e], st.stat_count[e], rr, false, tiles + (size_t)warp * n * D,
+                 out + (size_t)e * n * D);
 }
 
 // K5
@@ -1295,14 +1156,13 @@ __device__ void commit_episode_warp(const ebc_config &c, const ebc_state &st, in
     a0 = action[(size_t)e * 2];
     a1 = action[(size_t)e * 2 + 1];
   }
-  EpisodeHumans hm;
-  load_humans(c, st, e, H, lane, hm);
   const float4 rp = reinterpret_cast<const float4 *>(st.rob_pv)[e];
   const float4 rg = reinterpret_cast<const float4 *>(st.rob_gr)[e];
   const double theta = (double)st.rob_theta[e];
   const double gt = st.time[e];
+  EpisodeHumans hm;
   Outcome o;
-  evaluate_action_warp(c, st, e, lane, hm, rp, rg, theta, gt, a0, a1, o);
+  evaluate_action<32>(c, st, e, lane, H, rp, rg, theta, gt, a0, a1, hm, o);
   const double dt = c.time_step;
   // humans: agent.step(ActionXY), holonomic
 #pragma unroll
@@ -1370,33 +1230,26 @@ step_kernel(const ebc_config c, const ebc_state st, const double *__restrict__ a
   commit_episode_warp(c, st, e, lane, actions, action_idx, action, reward, done, event, dmin, dist_to_goal, sx);
 }
 
-// K1 + K2 fused, block per episode: every warp solves humans' LPs from the untouched state,
-// the block synchronises, then warp 0 commits.  One launch per env step on the policy-free path.
-// OBST: with ORCA obstacle half-planes (the episode's obstacle vertices staged in shared memory next to the
-// neighbour scratch); COMMIT = false is K1 alone in that block-per-episode shape (ebc_orca with obstacles).
-template <bool OBST, bool COMMIT, int GW>
+// K1 + K2 fused with ORCA obstacle half-planes, block per episode: the episode's obstacle vertices are staged in
+// shared memory next to the neighbour scratch, every warp solves humans' LPs from the untouched state, the block
+// synchronises, then warp 0 commits.  COMMIT = false is K1 alone in that shape (ebc_orca with obstacles).
+template <bool COMMIT>
 __global__ void __launch_bounds__(512)
 orca_step_kernel(const ebc_config c, const ebc_state st, const double *__restrict__ actions,
                  const int32_t *action_idx, const double *action, const uint8_t *active, double *reward,
                  uint8_t *done, uint8_t *event, double *dmin, double *dist_to_goal, const ebc_stats sx) {
-  constexpr int GPW = 32 / GW;       // humans per warp
-  __shared__ float scratch[16 * GPW][OBST ? OBST_SCRATCH_FLOATS : 32 * 5];
-  __shared__ __align__(16) ObstV so[OBST ? 64 : 1];
+  __shared__ float scratch[16][OBST_SCRATCH_FLOATS];
+  __shared__ __align__(16) ObstV so[64];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, n_warps = blockDim.x >> 5;
-  const int sub = lane / GW, gl = lane % GW;
   const int e = blockIdx.x;
   if (active && !active[e]) return;
   const int H = st.hum_count[e];
-  int V = 0;
-  if (OBST) {
-    V = stage_obstacles(c, st, e, so, threadIdx.x, blockDim.x);
-    __syncthreads();
-  }
-  const unsigned m = group_mask<GW>();
-  for (int h = warp * GPW + sub; h < H; h += n_warps * GPW) {
+  const int V = stage_obstacles(c, st, e, so, threadIdx.x, blockDim.x);
+  __syncthreads();
+  for (int h = warp; h < H; h += n_warps) {
     float nvx, nvy;
-    human_policy_warp<OBST, GW>(m, c, st, e, h, H, gl, scratch[warp * GPW + sub], nvx, nvy, so, V);
-    if (gl == 0)
+    human_policy_warp<true, 32>(FULL, c, st, e, h, H, lane, scratch[warp], nvx, nvy, so, V);
+    if (lane == 0)
       reinterpret_cast<float2 *>(st.hum_nv)[(size_t)e * c.max_humans + h] = make_float2(nvx, nvy);
   }
   if (!COMMIT) return;
@@ -1935,10 +1788,8 @@ static int orca_group(const ebc_sim *s) {
   if (s->cfg.orca_obstacles) return 32;
   return (s->cfg.max_humans + (s->cfg.robot_visible ? 1 : 0) <= 32 && s->cfg.orca_max_neighbors <= 16) ? 16 : 32;
 }
-static int fused_warps(const ebc_sim *s, int group) {
-  const int per_warp = 32 / group;
-  int warps = (s->cfg.max_humans + per_warp - 1) / per_warp;
-  warps = warps < 16 ? warps : 16;
+static int fused_warps(const ebc_sim *s) {   // orca_step_kernel: a warp per human, at most 16 warps per block
+  const int warps = s->cfg.max_humans < 16 ? s->cfg.max_humans : 16;
   return warps < 1 ? 1 : warps;
 }
 
@@ -1954,7 +1805,7 @@ static int launch_orca_groups(ebc_sim *s, const uint8_t *active, cudaStream_t st
 
 int ebc_launch_orca(ebc_sim *s, cudaStream_t stream) {
   if (s->cfg.orca_obstacles) {   // block per episode: the obstacle vertices are staged once per block
-    orca_step_kernel<true, false, 32><<<s->cfg.n_episodes, fused_warps(s, 32) * 32, 0, stream>>>(
+    orca_step_kernel<false><<<s->cfg.n_episodes, fused_warps(s) * 32, 0, stream>>>(
         s->cfg, s->st, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, ebc_stats{});
     return ebc_check_launch(s, "orca_step_kernel<obstacles, no commit>");
   }
@@ -1975,22 +1826,21 @@ int ebc_launch_lookahead(ebc_sim *s, float *vin, double *reward, uint8_t *done, 
                          cudaStream_t stream) {
   const long long pairs = (long long)s->cfg.n_episodes * s->cfg.n_actions;
   const int n = s->cfg.max_humans + s->cfg.max_statics, D = s->cfg.with_agent_type ? 17 : 13;
-  // small states: several (episode, action) pairs per warp (EBC_LOOKAHEAD_GROUP=32 forces one per warp)
-  const char *env = getenv("EBC_LOOKAHEAD_GROUP");
-  const int group = env ? atoi(env) : (n <= 8 ? 8 : (n <= 16 ? 16 : 32));
-  const int gpw = group == 8 || group == 16 ? 32 / group : 1;
+  // lanes per (episode, action): small states put several pairs in one warp
+  const int group = n <= 8 ? 8 : (n <= 16 ? 16 : 32);
+  const int gpw = 32 / group;
   const long long warps = (pairs + gpw - 1) / gpw;
   const int blocks = (int)((warps + EBC_WARPS_PER_BLOCK - 1) / EBC_WARPS_PER_BLOCK);
   const size_t smem = (size_t)EBC_WARPS_PER_BLOCK * gpw * n * D * sizeof(float);
   // without a destination for the rows the kernel leaves the robot part of every (episode, action) in s->d_la_rec:
   // K4's fused input path builds the rows from it (ebc_value with vin == NULL)
   float4 *rec = vin ? nullptr : s->d_la_rec;
-  if (group == 8 && n <= 8)
-    lookahead_group_kernel<8><<<blocks, EBC_THREADS, smem, stream>>>(s->cfg, s->st, s->d_actions, vin, reward, done, event, rec);
-  else if (group == 16 && n <= 16)
-    lookahead_group_kernel<16><<<blocks, EBC_THREADS, smem, stream>>>(s->cfg, s->st, s->d_actions, vin, reward, done, event, rec);
+  if (group == 8)
+    lookahead_kernel<8><<<blocks, EBC_THREADS, smem, stream>>>(s->cfg, s->st, s->d_actions, vin, reward, done, event, rec);
+  else if (group == 16)
+    lookahead_kernel<16><<<blocks, EBC_THREADS, smem, stream>>>(s->cfg, s->st, s->d_actions, vin, reward, done, event, rec);
   else
-    lookahead_kernel<<<blocks, EBC_THREADS, smem, stream>>>(s->cfg, s->st, s->d_actions, vin, reward, done, event, rec);
+    lookahead_kernel<32><<<blocks, EBC_THREADS, smem, stream>>>(s->cfg, s->st, s->d_actions, vin, reward, done, event, rec);
   s->la_rec_valid = rec != nullptr;
   return ebc_check_launch(s, "lookahead_kernel");
 }
@@ -2019,10 +1869,9 @@ int ebc_launch_step(ebc_sim *s, bool fused_orca, const int32_t *action_idx, cons
   if (fused_orca && s->cfg.orca_obstacles) {
     // block per episode: the obstacle vertices are staged in shared memory once, every warp solves humans' LPs,
     // the block synchronises, warp 0 commits
-    const int threads = fused_warps(s, 32) * 32;
-    orca_step_kernel<true, true, 32><<<s->cfg.n_episodes, threads, 0, stream>>>(s->cfg, s->st, s->d_actions, action_idx, action,
-                                                                              active, reward, done, event, dmin,
-                                                                              dist_to_goal, sx);
+    const int threads = fused_warps(s) * 32;
+    orca_step_kernel<true><<<s->cfg.n_episodes, threads, 0, stream>>>(s->cfg, s->st, s->d_actions, action_idx, action,
+                                                                    active, reward, done, event, dmin, dist_to_goal, sx);
     return ebc_check_launch(s, "orca_step_kernel");
   }
   if (fused_orca) {

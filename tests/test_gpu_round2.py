@@ -321,6 +321,42 @@ def test_half_warp_orca_is_bit_identical(oracle, H, S, R, dense, visible):
     assert np.array_equal(np_(out["16"][1]), r.hum_pv.numpy())
 
 
+@pytest.mark.parametrize("kin", ["holonomic", "unicycle"])
+def test_lookahead_group_widths_are_bit_identical(kin):
+    """K3 at every lane-group width on one batch: Hmax = 5, 13, 25 and 45 (+ 3 static slots) put a state's rows on groups
+    of 8, 16 and 32 lanes, the last with two humans per lane.  Outcomes, rows, the committed step and transform() are
+    equal bit for bit; the padding only appends zero rows."""
+    N, H, S, R = 1024, 5, 3, 3
+    cfg = random_cfg(kin, typed=True)
+    actions = build_action_space(0.8, kin)
+    batch = random_batch(N, H, S, R, seed=77)
+    idx = torch.as_tensor(np.random.default_rng(4).integers(0, 81, N), dtype=torch.int32, device="cuda:0")
+    out = []
+    for Hmax in (5, 13, 25, 45):
+        b = dict(batch)
+        for k in ("hum_pv", "hum_gr", "hum_type"):
+            pad = [(0, 0), (0, Hmax - H)] + [(0, 0)] * (b[k].ndim - 2)
+            b[k] = np.pad(b[k], pad)
+        g = BatchedSim(cfg, N, Hmax, S, R, 81, device="cuda:0")
+        g.set_actions(actions)
+        g.load_episodes(0, **b)
+        g.orca()
+        g.lookahead()
+        assert not g.vin[:, :, H + S:].any()
+        res = {k: getattr(g, k).clone() for k in ("la_reward", "la_done", "la_event")}
+        res["vin"] = g.vin[:, :, :H + S].clone()
+        g.step(action_idx=idx)
+        res.update({k: getattr(g, k).clone() for k in ("reward", "done", "event", "dmin", "rob_pv")})
+        res["hum_pv"] = g.hum_pv[:, :H].clone()
+        res["transform"] = g.transform()[:, :H + S].clone()
+        torch.cuda.synchronize()
+        out.append(res)
+        del g
+    for res in out[1:]:
+        for k, v in out[0].items():
+            assert np.array_equal(np_(res[k]).view(np.uint8), np_(v).view(np.uint8)), k
+
+
 @pytest.mark.parametrize("shape_name,N,kin,wname,typed", [
     ("CFG2", 1024, "holonomic", "weights_ebcadrl.npz", True),        # 16 rows per state: the transpose-reduce path
     ("CFG3", 2048, "unicycle", "weights_sarl_baseline.npz", False),  # 5 rows per state, D = 13, theta in the row
