@@ -116,7 +116,9 @@ __device__ void gemm_chunk(const float *in_s, int K, const float *__restrict__ w
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
         float x = acc[i][j] + b;
-        if (ep.gv) x += ep.gv[((ty * 8 + i) / ep.n_rows_per_state) * ep.gv_ld + col];
+        // with fewer than 4 rows per state the tile's MAX_TS states end before row 64: the rows past them belong to
+        // no state and their outputs are never read, but the index must stay inside GV
+        if (ep.gv) x += ep.gv[min((ty * 8 + i) / ep.n_rows_per_state, MAX_TS - 1) * ep.gv_ld + col];
         v[i] = (ep.relu && x < 0.0f) ? 0.0f : x;
       }
       *reinterpret_cast<float4 *>(out_s + col * LDA + ty * 8) = make_float4(v[0], v[1], v[2], v[3]);

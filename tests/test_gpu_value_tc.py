@@ -11,8 +11,9 @@ from ebc.engine import BatchedSim
 pytestmark = pytest.mark.gpu
 
 
-def torch_value(w, x, cnt, with_global=True):
-    """fp64 reference of the value network with ragged row counts."""
+def torch_value(w, x, cnt, with_global=True, return_weights=False):
+    """fp64 reference of the value network with ragged row counts.  `return_weights`: also return the softmax
+    attention weights [n_states, n] (0 on padding rows)."""
     W = {k: torch.as_tensor(v, device=x.device, dtype=torch.float64) for k, v in w.items()}
     n = x.shape[1]
 
@@ -31,7 +32,8 @@ def torch_value(w, x, cnt, with_global=True):
     wts = e / e.sum(1, keepdim=True)
     f = (wts[..., None] * h2).sum(1)
     j = torch.cat([xd[:, 0, :6], f], 1)
-    return lin(lin(lin(lin(j, "mlp3.0", True), "mlp3.2", True), "mlp3.4", True), "mlp3.6", False)[:, 0]
+    v = lin(lin(lin(lin(j, "mlp3.0", True), "mlp3.2", True), "mlp3.4", True), "mlp3.6", False)[:, 0]
+    return (v, wts) if return_weights else v
 
 
 def make_inputs(n_states, n, D, seed, ragged=True):
