@@ -60,21 +60,21 @@ template <int GW> __device__ __forceinline__ double grp_min_d(unsigned m, double
 // The group's ORCA lines: line index = lane + GW * chunk.  A group = the GW lanes that solve one agent's LP: the whole
 // warp (GW = 32), or a half warp (GW = 16: two agents per warp, every shuffle / ballot / reduction confined to the
 // half through its member mask `m`; `lane` is then the lane index inside the half).  LPL (lines per lane) = 1 on the
-// reference's live path (at most max_neighbors agent lines), 2 when obstacle half-planes are enabled (up to 64
-// lines, obstacle lines first; GW = 32 only).  Every function below is the same arithmetic for all (GW, LPL).
+// reference's live path (at most max_neighbors agent lines), 3 when obstacle half-planes are enabled (up to 96
+// lines: at most 64 obstacle lines first, then at most 32 agent lines; GW = 32 only).  Every function below is the
+// same arithmetic for all (GW, LPL).
 template <int LPL> struct Lines { Line l[LPL]; };
 
 template <int LPL, int GW>
 __device__ __forceinline__ void bcast_line(unsigned m, const Lines<LPL> &L, int i, float &px, float &py, float &dx,
                                            float &dy) {
-  const int il = i & (GW - 1);
-  if (LPL == 1 || i < GW) {
-    px = __shfl_sync(m, L.l[0].px, il, GW); py = __shfl_sync(m, L.l[0].py, il, GW);
-    dx = __shfl_sync(m, L.l[0].dx, il, GW); dy = __shfl_sync(m, L.l[0].dy, il, GW);
-  } else {
-    px = __shfl_sync(m, L.l[LPL - 1].px, il, GW); py = __shfl_sync(m, L.l[LPL - 1].py, il, GW);
-    dx = __shfl_sync(m, L.l[LPL - 1].dx, il, GW); dy = __shfl_sync(m, L.l[LPL - 1].dy, il, GW);
-  }
+  const int il = i & (GW - 1), ic = i / GW;
+  Line s = L.l[0];
+#pragma unroll
+  for (int c = 1; c < LPL; ++c)
+    if (ic == c) s = L.l[c];
+  px = __shfl_sync(m, s.px, il, GW); py = __shfl_sync(m, s.py, il, GW);
+  dx = __shfl_sync(m, s.dx, il, GW); dy = __shfl_sync(m, s.dy, il, GW);
 }
 
 // RVO2 linearProgram1 with the scan over earlier lines done by the lanes that hold them.
@@ -210,18 +210,23 @@ __device__ void lp3_warp(unsigned m, const Lines<LPL> &L, int lane, int n, int n
         Q.l[0].dx = __shfl_sync(m, P.l[0].dx, src, GW);
         Q.l[0].dy = __shfl_sync(m, P.l[0].dy, src, GW);
       } else {
-        const int m0 = __popc(vm[0]);
 #pragma unroll
         for (int c = 0; c < LPL; ++c) {
           const int t = lane + GW * c;                   // target index: the t-th surviving line
-          int sc = 0, sl = lane;
-          if (t < m0) { sc = 0; sl = (int)__fns(vm[0], 0, t + 1); }
-          else if (t < cnt) { sc = 1; sl = (int)__fns(vm[LPL - 1], 0, t - m0 + 1); }
-          const float a0 = __shfl_sync(m, P.l[0].px, sl, GW), a1 = __shfl_sync(m, P.l[LPL - 1].px, sl, GW);
-          const float b0 = __shfl_sync(m, P.l[0].py, sl, GW), b1 = __shfl_sync(m, P.l[LPL - 1].py, sl, GW);
-          const float c0 = __shfl_sync(m, P.l[0].dx, sl, GW), c1 = __shfl_sync(m, P.l[LPL - 1].dx, sl, GW);
-          const float d0 = __shfl_sync(m, P.l[0].dy, sl, GW), d1 = __shfl_sync(m, P.l[LPL - 1].dy, sl, GW);
-          Q.l[c].px = sc ? a1 : a0; Q.l[c].py = sc ? b1 : b0; Q.l[c].dx = sc ? c1 : c0; Q.l[c].dy = sc ? d1 : d0;
+          int sc = 0, sl = lane, base = 0;               // it sits in chunk sc, lane sl
+#pragma unroll
+          for (int k = 0; k < LPL; ++k) {
+            const int nk = __popc(vm[k]);
+            if (t >= base && t < base + nk) { sc = k; sl = (int)__fns(vm[k], 0, t - base + 1); }
+            base += nk;
+          }
+          Q.l[c] = Line{0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+          for (int k = 0; k < LPL; ++k) {
+            const float a = __shfl_sync(m, P.l[k].px, sl, GW), b = __shfl_sync(m, P.l[k].py, sl, GW);
+            const float d0 = __shfl_sync(m, P.l[k].dx, sl, GW), d1 = __shfl_sync(m, P.l[k].dy, sl, GW);
+            if (sc == k) { Q.l[c].px = a; Q.l[c].py = b; Q.l[c].dx = d0; Q.l[c].dy = d1; }
+          }
         }
       }
       const float tx = rx, ty = ry;
@@ -245,7 +250,7 @@ struct ObstV {                      // = ebc_obst_vertex, 48 bytes
   unsigned long long anc, anc_left, pad1;
 };
 static_assert(sizeof(ObstV) == sizeof(ebc_obst_vertex), "obstacle record layout");
-constexpr int OBST_SCRATCH_FLOATS = 64 * 4 + 16;   // per warp: 64 lines (or 32 x 5 neighbour floats) + 64 sorted ids
+constexpr int OBST_SCRATCH_FLOATS = 96 * 4 + 16;   // per warp: 96 lines (or 32 x 5 neighbour floats) + 64 sorted ids
 
 __device__ __forceinline__ float left_of(float ax, float ay, float bx, float by, float cx, float cy) {
   return det2(ax - cx, ay - cy, bx - ax, by - ay);
@@ -514,7 +519,7 @@ __device__ void orca_agent_warp(unsigned m, int lane, float px, float py, float 
                                 const bool (&cval)[2], int n_chunks, float neighbor_dist, int max_nb,
                                 float time_horizon, float time_step, float *scratch, float &outx, float &outy,
                                 const ObstV *so = nullptr, int V = 0, float th_obst = 0.0f) {
-  constexpr int LPL = OBST ? 2 : 1;
+  constexpr int LPL = OBST ? 3 : 1;
   static_assert(!OBST || GW == 32, "obstacle half-planes use the whole warp");
   // Agent::insertAgentNeighbor == keep the max_nb smallest (distSq, arrival index) below range
   float d[2];
@@ -613,12 +618,11 @@ __device__ void orca_agent_warp(unsigned m, int lane, float px, float py, float 
   Lines<LPL> L;
   int num_obst = 0;
   if (OBST) {
-    // obstacle lines first (Agent::computeNewVelocity), then the agent lines; at most 64 lines in all (the farthest
-    // agent neighbours are dropped beyond that -- RVO2 itself has no such bound)
+    // obstacle lines first (Agent::computeNewVelocity), then the agent lines: at most 64 + 32, all of them kept like
+    // RVO2 does
     Line *linebuf = reinterpret_cast<Line *>(scratch);
-    unsigned char *ids = reinterpret_cast<unsigned char *>(scratch + 64 * 4);
+    unsigned char *ids = reinterpret_cast<unsigned char *>(scratch + 96 * 4);
     num_obst = obstacle_lines_warp(so, V, lane, px, py, vx, vy, radius, max_speed, th_obst, linebuf, ids);
-    if (cnt > 64 - num_obst) cnt = 64 - num_obst;
     if (lane < cnt) linebuf[num_obst + lane] = A;
     __syncwarp(m);
 #pragma unroll

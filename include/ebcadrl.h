@@ -119,7 +119,10 @@ typedef struct ebc_config {
 /* Structure-of-arrays episode state.  The library BORROWS these arrays (owned by
  * the caller, e.g. torch tensors); it never frees them.  fp32 state, float4-packed
  * per agent so that one warp lane loads one agent with one 16-byte load.
- * Layout follows simulator/utils/state.py:1-92 (FullState / ObservableState). */
+ * Layout follows simulator/utils/state.py:1-92 (FullState / ObservableState).
+ * Slots past an episode's hum_count / stat_count / rect_count are neither read nor written by ebc_orca, ebc_robot_orca,
+ * ebc_lookahead, ebc_value, ebc_select, ebc_step, ebc_orca_step, ebc_transform or ebc_local_map_grid: the caller may
+ * leave anything there (ebc_reset and ebc_generate write whole episodes). */
 /* One RVO2 obstacle vertex (Obstacle.h: point_, unitDir_, nextObstacle_, prevObstacle_, isConvex_) plus this vertex's
  * place in RVO2's obstacle kd-tree (KdTree::buildObstacleTreeRecursive: one node per vertex, edges that straddle a
  * splitting line are split), from which every agent derives the tree's near-first visiting order for distance ties.
