@@ -310,6 +310,37 @@ int ebc_generate(ebc_sim *s, const ebc_scene_shape *shape, uint64_t seed, const 
   return ebc_launch_generate(s, shape, seed, episode_ids, mask, (cudaStream_t)stream);
 }
 
+int ebc_replay_scenes(ebc_sim *s, const ebc_replay_config *c, const uint32_t *seeds, const uint8_t *mask, double *poly_xy,
+                      int32_t *poly_count, int32_t *need, void *stream) {
+  REQUIRE_BOUND("ebc_replay_scenes");
+  if (!c || !seeds || !poly_count || !need || (c->max_polys > 0 && !poly_xy))
+    return ebc_fail(s, EBC_ERR_INVALID, "ebc_replay_scenes: null config, seeds or output");
+  for (int t = 0; t < 3; ++t)
+    if (c->count[t] < 0 || c->count[t] > 64)
+      return ebc_fail(s, EBC_ERR_INVALID, "ebc_replay_scenes: group %d holds %d agents (0..64)", t, c->count[t]);
+  const int r0 = c->rule[0], r1 = c->rule[1], r2 = c->rule[2];
+  if (r0 < EBC_REPLAY_SQUARE_CROSSING || r0 > EBC_REPLAY_ONE_STATIC ||     // scene_generator.py:589-591
+      (c->count[1] > 0 && r1 != EBC_REPLAY_SQUARE_CROSSING && r1 != EBC_REPLAY_CIRCLE_CROSSING &&
+       r1 != EBC_REPLAY_SQUARE_CROSSING_OLD) ||
+      (c->count[2] > 0 && r2 != EBC_REPLAY_SQUARE_CROSSING))
+    return ebc_fail(s, EBC_ERR_INVALID, "ebc_replay_scenes: rule (%d, %d, %d) does not exist for its list", r0, r1, r2);
+  if (c->num_circles < 0 || c->num_walls < 0 || c->max_polys < 0 || c->min_wall_length > c->max_wall_length ||
+      (c->num_walls > 0 && c->min_wall_length < 1))
+    return ebc_fail(s, EBC_ERR_INVALID, "ebc_replay_scenes: bad obstacle counts or wall lengths");
+  if (!(c->map_resolution > 0.0) || !(c->map_size_m > 0.0) || !(c->square_width >= 0.0) || !(c->circle_radius >= 0.0) ||
+      !(c->robot_radius >= 0.0) || !(c->discomfort_dist >= 0.0))
+    return ebc_fail(s, EBC_ERR_INVALID, "ebc_replay_scenes: sizes and distances must be non-negative, map size and resolution positive");
+  const double grid = rint(c->map_size_m / c->map_resolution);
+  if (c->num_circles + c->num_walls > 0 && !(grid >= 2.0 && grid <= 32767.0))
+    return ebc_fail(s, EBC_ERR_INVALID, "ebc_replay_scenes: a map of %.0f cells has no room for obstacles (2..32767)", grid);
+  if (c->randomize_attributes)          // agent.py:55: the drawn attributes must lie in (0, 20)
+    for (int t = 0; t < 3; ++t)
+      if (!(c->v_pref_min[t] > 0.0 && c->v_pref_max[t] < 20.0 && c->radius_min[t] > 0.0 && c->radius_max[t] < 20.0) &&
+          c->count[t] > 0)
+        return ebc_fail(s, EBC_ERR_INVALID, "ebc_replay_scenes: random attributes of group %d outside (0, 20)", t);
+  return ebc_launch_replay(s, c, seeds, mask, poly_xy, poly_count, need, (cudaStream_t)stream);
+}
+
 int ebc_local_map_angular(ebc_sim *s, const ebc_angular_map *map, const double *poly_xy, const int32_t *poly_count,
                           double *out, void *stream) {
   REQUIRE_BOUND("ebc_local_map_angular");

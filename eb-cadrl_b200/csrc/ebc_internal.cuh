@@ -122,6 +122,10 @@ int ebc_launch_grid_map(ebc_sim *s, const ebc_grid_map *map, uint8_t *out, cudaS
 int ebc_launch_generate(ebc_sim *s, const ebc_scene_shape *shape, uint64_t seed, const int64_t *episode_ids,
                         const uint8_t *mask, cudaStream_t st);
 
+// ebc_replay.cu
+int ebc_launch_replay(ebc_sim *s, const ebc_replay_config *cfg, const uint32_t *seeds, const uint8_t *mask,
+                      double *poly_xy, int32_t *poly_count, int32_t *need, cudaStream_t st);
+
 // ebc_value.cu
 int ebc_value_prepare(ebc_sim *s, const ebc_weights *w);
 void ebc_value_release(ebc_sim *s);

@@ -84,6 +84,22 @@ class EbcSceneShape(ctypes.Structure):
                 ("map_size_m", c_f64), ("map_resolution", c_f64), ("discomfort_dist", c_f64)]
 
 
+# EBC_REPLAY_* rule codes of ebc_replay_config, by the rule names of the [sim] section
+REPLAY_RULES = {"square_crossing": 0, "circle_crossing": 1, "mixed": 2, "mixed_20": 3, "one_static": 4,
+                "square_crossing_old": 5}
+REPLAY_RNG_SEED, REPLAY_RNG_RANDOM, REPLAY_RNG_UNIFORM, REPLAY_RNG_RANDINT, REPLAY_RNG_CHOICE_SIGN = range(5)
+
+
+class EbcReplayConfig(ctypes.Structure):     # one phase of simulator/scene/scene_generator.py (ebc_replay_scenes)
+    _fields_ = [("count", c_i32 * 3), ("rule", c_i32 * 3), ("randomize_attributes", c_i32),
+                ("num_circles", c_i32), ("num_walls", c_i32), ("min_wall_length", c_i32), ("max_wall_length", c_i32),
+                ("max_polys", c_i32), ("norm_fused", c_i32), ("reserved", c_i32),
+                ("v_pref", c_f64 * 3), ("radius", c_f64 * 3), ("v_pref_min", c_f64 * 3), ("v_pref_max", c_f64 * 3),
+                ("radius_min", c_f64 * 3), ("radius_max", c_f64 * 3),
+                ("square_width", c_f64), ("circle_radius", c_f64), ("discomfort_dist", c_f64),
+                ("robot_radius", c_f64), ("robot_v_pref", c_f64), ("map_size_m", c_f64), ("map_resolution", c_f64)]
+
+
 class EbcAngularMap(ctypes.Structure):       # [map] section of the env config (simulator/env.py:79-87)
     _fields_ = [("max_range", c_f64), ("min_angle", c_f64), ("max_angle", c_f64), ("dim", c_i32),
                 ("normalize", c_i32), ("max_polys", c_i32), ("reserved", c_i32)]
@@ -118,10 +134,14 @@ PROTOTYPES = {
     "ebc_transform": (c_i32, [SIM, vp, vp]),
     "ebc_reset": (c_i32, [SIM, ctypes.POINTER(EbcState), c_i32, vp, vp, vp]),
     "ebc_generate": (c_i32, [SIM, ctypes.POINTER(EbcSceneShape), ctypes.c_uint64, vp, vp, vp]),
+    "ebc_replay_scenes": (c_i32, [SIM, ctypes.POINTER(EbcReplayConfig), vp, vp, vp, vp, vp, vp]),
     "ebc_local_map_angular": (c_i32, [SIM, ctypes.POINTER(EbcAngularMap), vp, vp, vp, vp]),
     "ebc_local_map_grid": (c_i32, [SIM, ctypes.POINTER(EbcGridMap), vp, vp]),
     "ebc_debug_trace": (c_i32, [SIM, vp, c_i32]),
     "ebc_launch_count": (ctypes.c_int64, [SIM]),
+    "ebc_replay_scene_host": (c_i32, [ctypes.POINTER(EbcReplayConfig), ctypes.c_uint32, c_i32, c_i32, c_i32, vp, vp, vp,
+                                      vp, vp, vp, vp]),
+    "ebc_replay_rng_host": (c_i32, [vp, vp, c_i32, c_f64, c_f64, vp]),
 }
 
 LIB_PATH = os.environ.get("EBCADRL_LIB") or os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "lib",

@@ -1,12 +1,19 @@
 """BatchedEnv — N reference episodes at once: the batched face of simulator/env.py.
 
     env = BatchedEnv(env_config, policy, n_episodes, device)      # policy: rl.policy.sarl.SARL (configured)
-    env.reset_batch("test", seeds)         # env.reset x N   (host scene generator replaying the reference RNG)
+    env.reset_batch("test", seeds)         # env.reset x N   (the reference's seeded scenes, replayed in one launch)
     env.lookahead_batch()                  # onestep_lookahead x 81 x N  -> la_reward / la_event / vin
     env.step_batch(action_idx=...)         # env.step x N
     stats = env.run_episodes("test", seeds)                        # the Explorer's inner loop, on the device
 
 Episode r of rank k uses seed seeds[r]; sharding over ranks is the caller's slice of `seeds` (no collective).
+
+reset_batch builds every episode's scene on the device: ebc_replay_scenes replays numpy's seeded MT19937 stream and the
+scene generator's rules (simulator/scene/scene_generator.py, generate_random_scene with scene_number = seed) one thread
+per episode, and writes the humans, static discs, grid rectangles and obstacle polygons straight into the bound state.
+The host uploads the seeds and reads back one [N, 5] array of counts to check the capacity.  The host SceneGenerator
+still parses the INI (and serves the N = 1 env, simulator/env.py); its case counter advances as if it had generated
+the scenes.
 """
 import configparser
 
@@ -17,7 +24,7 @@ from . import abi
 from .actions import build_action_space
 from .config import SimConfig
 from .engine import BatchedSim
-from .scene import rects_from_zero_cells
+from .scene import replay_config, replay_rect_bound
 
 
 class _RobotStub(object):
@@ -70,7 +77,7 @@ class BatchedEnv(object):
 
     def __init__(self, env_config, policy=None, n_episodes=1, device="cuda:0", max_humans=None, max_statics=None,
                  max_rects=None):
-        from simulator.scene.scene_generator import SceneGenerator   # host scene generation (reference RNG)
+        from simulator.scene.scene_generator import SceneGenerator   # the INI's scene settings (and the case counter)
         if not isinstance(env_config, configparser.RawConfigParser):
             cp = configparser.RawConfigParser()
             cp.read(env_config)
@@ -83,6 +90,7 @@ class BatchedEnv(object):
             self.cfg.with_agent_type = bool(getattr(policy, "with_agent_type", False))
             self.cfg.gamma = policy.gamma or self.cfg.gamma
         self.scene = SceneGenerator(env_config)
+        self._replay_configs = {}      # ebc_replay_config per (phase, multiagent_training, list sizes)
         self.robot = _RobotStub(env_config, policy if policy is not None else type("P", (), dict(
             multiagent_training=True, name="none", kinematics="holonomic"))())
         self.cfg.robot_visible = self.robot.visible
@@ -94,7 +102,8 @@ class BatchedEnv(object):
         walls, circles = sg.num_walls or 0, sg.num_circles or 0
         discs_per_wall = int(np.ceil(sg.max_wall_length / np.sqrt(2.0)))
         S = max_statics if max_statics is not None else walls * discs_per_wall + circles
-        R = max_rects if max_rects is not None else 4 * (walls + circles)
+        # the replay's per-obstacle rectangles: one per obstacle inside the map, a lattice for a striped border patch
+        R = max_rects if max_rects is not None else replay_rect_bound(sg)
         self.N = n_episodes
         n_actions = policy.n_actions if policy is not None and hasattr(policy, "n_actions") else 81
         self.sim = BatchedSim(self.cfg, n_episodes, H, S, R, n_actions, device=device)
@@ -164,48 +173,40 @@ class BatchedEnv(object):
 
     # ---- env.reset x N ---------------------------------------------------------------------------------
     def reset_batch(self, phase, seeds):
-        """seeds[e] = scene_number of episode e (the reference: counter offset + case counter, or explicit)."""
+        """seeds[e] = scene_number of episode e (the reference: counter offset + case counter, or explicit): the scene
+        generate_random_scene(phase, scene_number = seeds[e]) makes, regenerated on the device in one launch.
+
+        A scene that does not fit the batch's capacity (humans, static discs, grid rectangles) raises EbcError naming
+        its seed.  The check needs the kernel's counts, so by then every episode's state in the sim has been
+        overwritten (the oversized scenes truncated): reset again before stepping.  self.poly_xy / poly_count and the
+        scene generator's counters are left as they were."""
         sim, sg = self.sim, self.scene
         assert len(seeds) == self.N
-        H, S, R = sim.Hmax, max(sim.Smax, 1), max(sim.Rmax, 1)
-        pv = np.zeros((self.N, H, 4), np.float32); gr = np.zeros((self.N, H, 4), np.float32)
-        ty = np.zeros((self.N, H), np.uint8); hc = np.zeros(self.N, np.int32)
-        sd = np.zeros((self.N, S, 4), np.float32); sc = np.zeros(self.N, np.int32)
-        rc = np.zeros((self.N, R, 4), np.int16); rcc = np.zeros(self.N, np.int32)
+        seeds = np.asarray([int(x) for x in seeds], dtype=object)
+        bad = [int(x) for x in seeds if not 0 <= int(x) <= 0xFFFFFFFF]
+        if bad:
+            raise ValueError("Seed must be between 0 and 2**32 - 1 (got %d)" % bad[0])      # np.random.seed's bound
+        seeds = seeds.astype(np.uint32)
+        multi = bool(self.robot.policy.multiagent_training)
+        key = (phase, multi, sg.adult_num, sg.bicycle_num, sg.children_num)
+        if key not in self._replay_configs:
+            self._replay_configs[key] = replay_config(sg, phase, multi, max((sg.num_circles or 0) + (sg.num_walls or 0), 1))
+        cfg = self._replay_configs[key]
         rad = sg.circle_radius
-        polys = []
-        for e, seed in enumerate(seeds):
-            self.robot.set(0, -rad, 0, rad, 0, 0, np.pi / 2)
-            sg.generate_random_scene(self.COUNTER_OFFSET, phase, scene_number=int(seed))
-            hs = sg.adults + sg.bicycles + sg.children
-            if len(hs) > sim.Hmax or len(sg.static_obstacles_as_pedestrians) > sim.Smax:
-                raise abi.EbcError("scene %d exceeds the batch capacity (H=%d, S=%d)" % (
-                    seed, len(hs), len(sg.static_obstacles_as_pedestrians)))
-            for i, h in enumerate(hs):
-                pv[e, i] = (h.px, h.py, h.vx, h.vy)
-                gr[e, i] = (h.gx, h.gy, h.v_pref, h.radius)
-                ty[e, i] = int(h.agent_type)
-            hc[e] = len(hs)
-            for i, s in enumerate(sg.static_obstacles_as_pedestrians):
-                sd[e, i, :3] = (s.px, s.py, s.radius)
-            sc[e] = len(sg.static_obstacles_as_pedestrians)
-            rects = rects_from_zero_cells(sg.map == 0)
-            if len(rects) > sim.Rmax:
-                raise abi.EbcError("scene %d needs %d grid rectangles (capacity %d)" % (seed, len(rects), sim.Rmax))
-            rc[e, :len(rects)] = rects
-            rcc[e] = len(rects)
-            polys.append(np.asarray(sg.obstacle_vertices, dtype=np.float64).reshape(-1, 4, 2))
-        # scene.obstacle_vertices of every episode, for the angular local map (local_map_batch)
-        P = max([len(v) for v in polys] + [1])
-        xy = np.zeros((self.N, P, 4, 2), np.float64)
-        for e, v in enumerate(polys):
-            xy[e, :len(v)] = v
-        self.poly_xy = torch.as_tensor(xy).to(self.device)
-        self.poly_count = torch.as_tensor(np.array([len(v) for v in polys], np.int32)).to(self.device)
-        rob_pv = np.tile(np.array([0, -rad, 0, 0], np.float32), (self.N, 1))
-        rob_gr = np.tile(np.array([0, rad, self.robot.v_pref, self.robot.radius], np.float32), (self.N, 1))
-        sim.load_episodes(0, pv, gr, ty, hc, sd, sc, rc, rcc, rob_pv, rob_gr,
-                          np.full(self.N, np.pi / 2, np.float32), np.zeros(self.N))
+        self.robot.set(0, -rad, 0, rad, 0, 0, np.pi / 2)
+        dev_seeds = torch.from_numpy(seeds.view(np.int32)).to(self.device)
+        poly_xy, poly_count, need = sim.replay_scenes(cfg, dev_seeds)
+        need = need.cpu().numpy()
+        for e in np.nonzero((need[:, 0] > sim.Hmax) | (need[:, 1] > sim.Smax) | (need[:, 2] > sim.Rmax))[0][:1]:
+            if need[e, 0] > sim.Hmax or need[e, 1] > sim.Smax:
+                raise abi.EbcError("scene %d exceeds the batch capacity (H=%d, S=%d)" % (seeds[e], need[e, 0], need[e, 1]))
+            raise abi.EbcError("scene %d needs %d grid rectangles (capacity %d)" % (seeds[e], need[e, 2], sim.Rmax))
+        self.poly_xy, self.poly_count = poly_xy, poly_count
+        # what the host generator leaves behind: the case counter advanced once per scene, and the adult count the
+        # mixed rules draw (the last scene's)
+        sg.case_counter[phase] = (sg.case_counter[phase] + self.N) % sg.case_size[phase]
+        if self.N and cfg.rule[0] in (abi.REPLAY_RULES["mixed"], abi.REPLAY_RULES["mixed_20"]):
+            sg.adult_num = int(need[-1, 4])
 
     # ---- thin batched calls ------------------------------------------------------------------------------
     def lookahead_batch(self):

@@ -342,6 +342,25 @@ class BatchedSim(object):
         self.be.call("generate", self.h, ctypes.byref(shape.to_abi()), ctypes.c_uint64(synth.SEED_BASE if seed is None else seed),
                      _ptr(episode_ids), _ptr(mask), stream=self._stream())
 
+    def replay_scenes(self, config, seeds, mask=None, poly_xy=None, poly_count=None, need=None):
+        """env.reset with the REFERENCE's seeded scene for the masked episodes: generate_random_scene(scene_number =
+        seeds[e]) replayed on the device (ebc_replay_scenes), `config` an abi.EbcReplayConfig (ebc.scene.replay_config),
+        `seeds` an int32 device tensor holding the uint32 seeds' bits.  Returns device tensors poly_xy [N, Pmax, 4, 2]
+        float64 (scene.obstacle_vertices), poly_count [N] int32 and need [N, 5] int32 (humans, static discs, grid
+        rectangles and polygons the scene holds, then the adult count its rule left); a count above the capacity means
+        the scene did not fit.  Pass the three outputs to keep the masked-off episodes' entries of earlier calls."""
+        assert seeds.dtype == torch.int32 and seeds.shape == (self.N,) and seeds.device == self.device
+        P = int(config.max_polys)
+        z = lambda *shape, dtype: torch.zeros(*shape, dtype=dtype, device=self.device)  # noqa: E731
+        poly_xy = z(self.N, max(P, 1), 4, 2, dtype=torch.float64) if poly_xy is None else poly_xy
+        poly_count = z(self.N, dtype=torch.int32) if poly_count is None else poly_count
+        need = z(self.N, 5, dtype=torch.int32) if need is None else need
+        assert tuple(poly_xy.shape) == (self.N, max(P, 1), 4, 2) and poly_xy.dtype == torch.float64 and poly_xy.is_contiguous()
+        assert tuple(need.shape) == (self.N, 5) and need.dtype == torch.int32 and poly_count.dtype == torch.int32
+        self.be.call("replay_scenes", self.h, ctypes.byref(config), _ptr(seeds), _ptr(mask), _ptr(poly_xy), _ptr(poly_count),
+                     _ptr(need), stream=self._stream())
+        return poly_xy, poly_count, need
+
     def reset(self, pool, pool_index=None, mask=None):
         """env.reset for the masked episodes from a device scene pool (simulator/env.py:128-205)."""
         self.be.call("reset", self.h, ctypes.byref(pool.state), pool.size, _ptr(pool_index), _ptr(mask),

@@ -3,8 +3,9 @@
 A restatement of simulator/scene/scene_generator.py that REPLAYS THE REFERENCE'S numpy RNG STREAM
 (np.random.seed(seed) then the same draws in the same order), so that for a given seed the agents, the
 occupancy grid and the static discs are identical to the reference's (pinned by tests/golden/scenes.npz).
-Scene generation runs once per episode on the host and is not a kernel (SURVEY §8f-1); throughput runs use
-the counter-based generator in ebc/synth.py instead.
+The N = 1 env generates its scenes here, once per episode; BatchedEnv.reset_batch replays this module on the device
+(ebc_replay_scenes, csrc/ebc_replay.cu), held to it bit for bit by tests/test_scene_replay.py; throughput runs use the
+counter-based generator in ebc/synth.py instead.
 
 Crossing rules: square_crossing (:672-712), circle_crossing (:593-650), mixed (:523-577), mixed_20
 (:466-501,578-582), one_static (:583-589).  Static map: walls/circles (:113-290), grid (:888-922),

@@ -357,6 +357,58 @@ typedef struct ebc_scene_shape {
 int ebc_generate(ebc_sim *sim, const ebc_scene_shape *shape, uint64_t seed, const int64_t *episode_ids,
                  const uint8_t *mask, void *stream);
 
+/* The reference's OWN seeded scenes on the device: generate_random_scene(scene_number = seed)
+ * (simulator/scene/scene_generator.py:330-378) replayed for every episode e with mask[e] != 0 (mask NULL = all), one
+ * thread per episode.  np.random.seed(seeds[e]) (:362) seeds numpy's legacy MT19937 (init_genrand), and every draw
+ * follows in the reference's order, rejected tries included: adults by their rule (:503-591; square_crossing :672-712,
+ * circle_crossing :593-618, mixed :523-577, mixed_20 :492-501,578-582, one_static :583-589), then bicycles
+ * (square_crossing_old :714-761), then children, then circles and walls (:292-328).  Agent attributes are drawn
+ * (v_pref, then radius, simulator/agents/agent.py:49-56) when randomize_attributes is set.  The arithmetic is the
+ * reference's float64 sequence, narrowed to fp32 at the store.  The one operation not bit-for-bit the host's is
+ * circle_crossing's double cos / sin: CUDA's and the host libm's need not round alike.  On the tested seeds they always
+ * agreed, but a last-bit difference is not bounded in its effect: it feeds the following too_close tests, can flip an
+ * accept / reject decision, and then changes every later draw of that scene.
+ * Writes what BatchedEnv.reset_batch loads: humans (adults, bicycles, children, at rest; hum_nv cleared), the static
+ * discs (:380-422), the grid's zero cells (:888-922) as rectangles -- an obstacle strictly inside the map is one
+ * rectangle; one on the border, where the per-cell path writes the product of two per-axis cell sets (every other cell
+ * along an axis of odd size: Python's half-to-even rounding), is one rectangle per pair of per-axis runs --, the robot
+ * at (0, -R) -> (0, R) at rest facing +y, time = 0.  Slots past the scene's counts are zeroed; nothing is written past
+ * Hmax / Smax / Rmax / max_polys.
+ *   poly_xy    [N*max_polys*4*2] f64 (device): scene.obstacle_vertices, circles then walls, 4 vertices each
+ *   poly_count [N] i32 (device)
+ *   need       [N*5] i32 (device): humans, static discs, rectangles and polygons the scene holds (a count above the
+ *              capacity means the scene did not fit), then the adult count: for the mixed rules the one they draw and leave
+ *              in SceneGenerator.adult_num (:537,580), otherwise the adult list's configured size
+ *   seeds      [N] u32 (device) */
+enum {
+  EBC_REPLAY_SQUARE_CROSSING = 0,      /* adults, bicycles, children */
+  EBC_REPLAY_CIRCLE_CROSSING = 1,      /* adults, bicycles */
+  EBC_REPLAY_MIXED = 2,                /* adults */
+  EBC_REPLAY_MIXED_20 = 3,             /* adults */
+  EBC_REPLAY_ONE_STATIC = 4,           /* adults */
+  EBC_REPLAY_SQUARE_CROSSING_OLD = 5   /* bicycles */
+};
+typedef struct ebc_replay_config {     /* one phase of SceneGenerator (scene_generator.py:26-66) */
+  int32_t count[3];                    /* adults, bicycles, children (1 each in train / val without multiagent_training) */
+  int32_t rule[3];                     /* EBC_REPLAY_* of each list (the phase's train_val_sim_* or test_sim_*) */
+  int32_t randomize_attributes;        /* [env] randomize_attributes */
+  int32_t num_circles, num_walls;      /* [map] */
+  int32_t min_wall_length, max_wall_length;
+  int32_t max_polys;                   /* Pmax: polygon slots per episode in poly_xy */
+  int32_t norm_fused;                  /* 1: numpy.linalg.norm((x, y)) of the numpy being matched is
+                                          sqrt(fma(y, y, x * x)) (OpenBLAS ddot on FMA-capable x86 cores);
+                                          0: sqrt(x * x + y * y) */
+  int32_t reserved;
+  double v_pref[3], radius[3];         /* [adults] [bicycles] [children] v_pref / radius (used unless drawn) */
+  double v_pref_min[3], v_pref_max[3], radius_min[3], radius_max[3];
+  double square_width, circle_radius;  /* [sim] */
+  double discomfort_dist;              /* [reward] discomfort_dist */
+  double robot_radius, robot_v_pref;   /* [robot] */
+  double map_size_m, map_resolution;   /* [map] */
+} ebc_replay_config;
+int ebc_replay_scenes(ebc_sim *sim, const ebc_replay_config *cfg, const uint32_t *seeds, const uint8_t *mask,
+                      double *poly_xy, int32_t *poly_count, int32_t *need, void *stream);
+
 /* Angular local map of simulator/env.py:468-628 (SURVEY 8f-3): for every episode the distance to the closest
  * obstacle outline in each of `dim` angular sectors around the robot, in the robot's heading frame (angle 0 at
  * the negative x axis as in the reference), clipped to max_range and optionally normalised by it.  What
@@ -404,6 +456,17 @@ int ebc_local_map_grid(ebc_sim *sim, const ebc_grid_map *map, uint8_t *out, void
 int ebc_debug_trace(ebc_sim *sim, long long *out, int32_t n);
 /* Number of kernels this handle has launched so far (bench.py's gpu_launches). */
 int64_t ebc_launch_count(const ebc_sim *sim);
+/* The scene replay of ebc_replay_scenes on the HOST, same function, for one seed: host arrays of max_humans /
+ * max_statics / max_rects / cfg->max_polys slots in the ebc_state layout, need [5].  No handle, no device. */
+int ebc_replay_scene_host(const ebc_replay_config *cfg, uint32_t seed, int32_t max_humans, int32_t max_statics,
+                          int32_t max_rects, float *hum_pv, float *hum_gr, uint8_t *hum_type, float *stat, int16_t *rect,
+                          double *poly_xy, int32_t *need);
+/* One numpy primitive of the replay on a given MT19937 state (key [624], pos, as numpy's get_state() holds them),
+ * advanced in place: seed(a), random(), uniform(a, b), randint(a, b) (bounds truncated toward zero like numpy's), or
+ * choice([1, -1], p=[0.5, 0.5]).  The result goes to *out. */
+enum { EBC_REPLAY_RNG_SEED = 0, EBC_REPLAY_RNG_RANDOM = 1, EBC_REPLAY_RNG_UNIFORM = 2, EBC_REPLAY_RNG_RANDINT = 3,
+       EBC_REPLAY_RNG_CHOICE_SIGN = 4 };
+int ebc_replay_rng_host(uint32_t *key, int32_t *pos, int32_t op, double a, double b, double *out);
 #endif
 
 /* ---- CPU twins (oracle/libebc_oracle.so only; HOST pointers; test infrastructure) -- */
