@@ -341,6 +341,16 @@ int ebc_replay_scenes(ebc_sim *s, const ebc_replay_config *c, const uint32_t *se
   return ebc_launch_replay(s, c, seeds, mask, poly_xy, poly_count, need, (cudaStream_t)stream);
 }
 
+int ebc_build_obstacles(ebc_sim *s, const double *poly_xy, const int32_t *poly_count, int32_t max_polys,
+                        const uint8_t *mask, int32_t *need, void *stream) {
+  REQUIRE_BOUND("ebc_build_obstacles");
+  if (!s->cfg.orca_obstacles || s->cfg.max_obst < 1)
+    return ebc_fail(s, EBC_ERR_INVALID, "ebc_build_obstacles: needs cfg.orca_obstacles and max_obst >= 1");
+  if (!poly_count || !need || max_polys < 0 || (max_polys > 0 && !poly_xy))
+    return ebc_fail(s, EBC_ERR_INVALID, "ebc_build_obstacles: null polygons or output, or max_polys < 0");
+  return ebc_launch_build_obstacles(s, poly_xy, poly_count, max_polys, mask, need, (cudaStream_t)stream);
+}
+
 int ebc_local_map_angular(ebc_sim *s, const ebc_angular_map *map, const double *poly_xy, const int32_t *poly_count,
                           double *out, void *stream) {
   REQUIRE_BOUND("ebc_local_map_angular");

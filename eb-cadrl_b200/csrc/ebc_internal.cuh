@@ -126,6 +126,10 @@ int ebc_launch_generate(ebc_sim *s, const ebc_scene_shape *shape, uint64_t seed,
 int ebc_launch_replay(ebc_sim *s, const ebc_replay_config *cfg, const uint32_t *seeds, const uint8_t *mask,
                       double *poly_xy, int32_t *poly_count, int32_t *need, cudaStream_t st);
 
+// ebc_obstacles.cu
+int ebc_launch_build_obstacles(ebc_sim *s, const double *poly_xy, const int32_t *poly_count, int max_polys,
+                               const uint8_t *mask, int32_t *need, cudaStream_t st);
+
 // ebc_value.cu
 int ebc_value_prepare(ebc_sim *s, const ebc_weights *w);
 void ebc_value_release(ebc_sim *s);

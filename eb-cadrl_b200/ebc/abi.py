@@ -135,6 +135,7 @@ PROTOTYPES = {
     "ebc_reset": (c_i32, [SIM, ctypes.POINTER(EbcState), c_i32, vp, vp, vp]),
     "ebc_generate": (c_i32, [SIM, ctypes.POINTER(EbcSceneShape), ctypes.c_uint64, vp, vp, vp]),
     "ebc_replay_scenes": (c_i32, [SIM, ctypes.POINTER(EbcReplayConfig), vp, vp, vp, vp, vp, vp]),
+    "ebc_build_obstacles": (c_i32, [SIM, vp, vp, c_i32, vp, vp, vp]),
     "ebc_local_map_angular": (c_i32, [SIM, ctypes.POINTER(EbcAngularMap), vp, vp, vp, vp]),
     "ebc_local_map_grid": (c_i32, [SIM, ctypes.POINTER(EbcGridMap), vp, vp]),
     "ebc_debug_trace": (c_i32, [SIM, vp, c_i32]),

@@ -11,11 +11,14 @@ Episode r of rank k uses seed seeds[r]; sharding over ranks is the caller's slic
 reset_batch builds every episode's scene on the device: ebc_replay_scenes replays numpy's seeded MT19937 stream and the
 scene generator's rules (simulator/scene/scene_generator.py, generate_random_scene with scene_number = seed) one thread
 per episode, and writes the humans, static discs, grid rectangles and obstacle polygons straight into the bound state.
-The host uploads the seeds and reads back one [N, 5] array of counts to check the capacity.  The host SceneGenerator
+With the env INI's `[sim] orca_obstacles = true` (this project's key; off by default, like the reference) the humans
+avoid walls: ebc_build_obstacles turns the polygons into RVO2 obstacle records on the device right after the replay.
+The host uploads the seeds and reads back one array of counts to check the capacity.  The host SceneGenerator
 still parses the INI (and serves the N = 1 env, simulator/env.py); its case counter advances as if it had generated
 the scenes.
 """
 import configparser
+import dataclasses
 
 import numpy as np
 import torch
@@ -47,7 +50,8 @@ class TargetValue(object):
 
     def __init__(self, env):
         sim = env.sim
-        self.sim = BatchedSim(env.cfg, 1, sim.Hmax, sim.Smax, 0, sim.A, device=sim.device)
+        cfg = dataclasses.replace(env.cfg, orca_obstacles=False)       # runs K4 only: no obstacle slots needed
+        self.sim = BatchedSim(cfg, 1, sim.Hmax, sim.Smax, 0, sim.A, device=sim.device)
         self.value_mode = getattr(env.policy, "value_mode", None)
 
     def set_model(self, model):
@@ -76,7 +80,7 @@ class BatchedEnv(object):
     COUNTER_OFFSET = {"train": 2000, "val": 0, "test": 1000}     # env.py:153-158
 
     def __init__(self, env_config, policy=None, n_episodes=1, device="cuda:0", max_humans=None, max_statics=None,
-                 max_rects=None):
+                 max_rects=None, max_obst=None):
         from simulator.scene.scene_generator import SceneGenerator   # the INI's scene settings (and the case counter)
         if not isinstance(env_config, configparser.RawConfigParser):
             cp = configparser.RawConfigParser()
@@ -104,9 +108,11 @@ class BatchedEnv(object):
         S = max_statics if max_statics is not None else walls * discs_per_wall + circles
         # the replay's per-obstacle rectangles: one per obstacle inside the map, a lattice for a striped border patch
         R = max_rects if max_rects is not None else replay_rect_bound(sg)
+        # [sim] orca_obstacles: RVO2 obstacle records of the scene's polygons, built on the device at every reset
+        O = max_obst if max_obst is not None else (64 if self.cfg.orca_obstacles else 0)
         self.N = n_episodes
         n_actions = policy.n_actions if policy is not None and hasattr(policy, "n_actions") else 81
-        self.sim = BatchedSim(self.cfg, n_episodes, H, S, R, n_actions, device=device)
+        self.sim = BatchedSim(self.cfg, n_episodes, H, S, R, n_actions, device=device, max_obst=O)
         self.device = self.sim.device
         if policy is not None:
             if policy.action_space is None:
@@ -176,9 +182,13 @@ class BatchedEnv(object):
         """seeds[e] = scene_number of episode e (the reference: counter offset + case counter, or explicit): the scene
         generate_random_scene(phase, scene_number = seeds[e]) makes, regenerated on the device in one launch.
 
-        A scene that does not fit the batch's capacity (humans, static discs, grid rectangles) raises EbcError naming
-        its seed.  The check needs the kernel's counts, so by then every episode's state in the sim has been
-        overwritten (the oversized scenes truncated): reset again before stepping.  self.poly_xy / poly_count and the
+        With [sim] orca_obstacles set, the scene's polygons then become RVO2 obstacle records on the device
+        (ebc_build_obstacles), before the one readback of the counts.
+
+        A scene that does not fit the batch's capacity (humans, static discs, grid rectangles, obstacle records) raises
+        EbcError naming its seed; polygons are never dropped to make a scene fit.  The check needs the kernel's counts,
+        so by then every episode's state in the sim has been overwritten (the oversized scenes truncated): reset again
+        before stepping.  self.poly_xy / poly_count and the
         scene generator's counters are left as they were."""
         sim, sg = self.sim, self.scene
         assert len(seeds) == self.N
@@ -196,11 +206,16 @@ class BatchedEnv(object):
         self.robot.set(0, -rad, 0, rad, 0, 0, np.pi / 2)
         dev_seeds = torch.from_numpy(seeds.view(np.int32)).to(self.device)
         poly_xy, poly_count, need = sim.replay_scenes(cfg, dev_seeds)
+        if self.cfg.orca_obstacles:
+            need = torch.cat([need, sim.build_obstacles(poly_xy, poly_count)[:, None]], 1)
         need = need.cpu().numpy()
-        for e in np.nonzero((need[:, 0] > sim.Hmax) | (need[:, 1] > sim.Smax) | (need[:, 2] > sim.Rmax))[0][:1]:
+        obst_bad = need[:, 5] < 0 if self.cfg.orca_obstacles else np.zeros(self.N, bool)
+        for e in np.nonzero((need[:, 0] > sim.Hmax) | (need[:, 1] > sim.Smax) | (need[:, 2] > sim.Rmax) | obst_bad)[0][:1]:
             if need[e, 0] > sim.Hmax or need[e, 1] > sim.Smax:
                 raise abi.EbcError("scene %d exceeds the batch capacity (H=%d, S=%d)" % (seeds[e], need[e, 0], need[e, 1]))
-            raise abi.EbcError("scene %d needs %d grid rectangles (capacity %d)" % (seeds[e], need[e, 2], sim.Rmax))
+            if need[e, 2] > sim.Rmax:
+                raise abi.EbcError("scene %d needs %d grid rectangles (capacity %d)" % (seeds[e], need[e, 2], sim.Rmax))
+            raise abi.EbcError("scene %d needs more than %d ORCA obstacle records" % (seeds[e], sim.Omax))
         self.poly_xy, self.poly_count = poly_xy, poly_count
         # what the host generator leaves behind: the case counter advanced once per scene, and the adult count the
         # mixed rules draw (the last scene's)

@@ -1,7 +1,11 @@
 """INI -> ebc_config.  Key names and fallbacks are the reference's, verbatim:
 simulator/env.py:58-87, simulator/utils/reward.py:18-75, simulator/scene/scene_generator.py:26-72,
 simulator/agents/agent.py:16-34, rl/policy/cadrl.py:73-82, rl/policy/sarl.py:90-128,
-simulator/policy/orca.py:57-69 (SURVEY Appendix D)."""
+simulator/policy/orca.py:57-69 (SURVEY Appendix D).
+
+One key is this project's own: `[sim] orca_obstacles` (boolean, default false).  With it set, humans (and the ORCA
+robot of imitation learning) avoid the scene's obstacle polygons with RVO2's obstacle half-planes.  The reference
+does not read it, so an INI that sets it still runs there unchanged, with humans that walk through walls."""
 import configparser
 from dataclasses import dataclass, field
 from typing import List
@@ -76,6 +80,9 @@ class SimConfig:
         c.robot_visible = g.getboolean("robot", "visible")
         c.human_policy = [g.get(sec, "policy", fallback="orca") if g.has_section(sec) else "orca"
                           for sec in ("adults", "bicycles", "children")]
+        # this project's key, not the reference's: walls-aware humans (SURVEY 8f-4).  The reference's RawConfigParser
+        # ignores it, so the same INI still runs there, with humans that ignore walls.
+        c.orca_obstacles = g.getboolean("sim", "orca_obstacles", fallback=False)
         if policy_config is not None:
             p = policy_config
             c.gamma = p.getfloat("rl", "gamma")

@@ -361,6 +361,20 @@ class BatchedSim(object):
                      _ptr(need), stream=self._stream())
         return poly_xy, poly_count, need
 
+    def build_obstacles(self, poly_xy, poly_count, mask=None):
+        """RVO2's obstacle records of every masked episode from its polygons (ebc_build_obstacles, SURVEY 8f-4): what
+        orca_obstacles.py's addObstacle + processObstacles make of scene.obstacle_vertices, written into obst /
+        obst_count on the device.  `poly_xy` [N, Pmax, 4, 2] float64 and `poly_count` [N] int32 as replay_scenes
+        returns them.  Returns need [N] int32 on the device: the records each episode needs, -1 where the kd-tree's
+        edge splitting overflows Omax (obst_count is then 0); 0 for masked-off episodes."""
+        assert poly_xy.dtype == torch.float64 and poly_xy.dim() == 4 and tuple(poly_xy.shape[2:]) == (4, 2)
+        assert poly_xy.shape[0] == self.N and poly_xy.is_contiguous()
+        assert poly_count.dtype == torch.int32 and tuple(poly_count.shape) == (self.N,)
+        need = torch.zeros(self.N, dtype=torch.int32, device=self.device)
+        self.be.call("build_obstacles", self.h, _ptr(poly_xy), _ptr(poly_count), poly_xy.shape[1], _ptr(mask), _ptr(need),
+                     stream=self._stream())
+        return need
+
     def reset(self, pool, pool_index=None, mask=None):
         """env.reset for the masked episodes from a device scene pool (simulator/env.py:128-205)."""
         self.be.call("reset", self.h, ctypes.byref(pool.state), pool.size, _ptr(pool_index), _ptr(mask),

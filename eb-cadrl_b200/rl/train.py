@@ -7,7 +7,11 @@ same artefacts (`output.log`, `il_model.pth`, `rl_model_{episode}.pth`, configs 
 What changed versus the reference: the 8-process pool (rl/utils/parallel_explorer.py) is a batch of
 `--episodes_per_iter` episodes per GPU on the device; with W ranks every rank samples its own seeds, the
 value-network gradient is all-reduced over NCCL once per optimizer step and the evaluation counters are
-all-gathered.  Replay memory, optimizer state and epsilon are not checkpointed (like the reference)."""
+all-gathered.  Replay memory, optimizer state and epsilon are not checkpointed (like the reference).
+
+Walls-aware humans come from the env INI, not a flag: with `[sim] orca_obstacles = true` (this project's key, off by
+default like the reference) humans avoid the scene's walls, and so does the ORCA robot that imitation learning
+follows (ebc_robot_orca).  rl.test and rl.test_parallel read the same key from the env INI they are given."""
 import argparse
 import configparser
 import copy

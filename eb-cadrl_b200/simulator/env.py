@@ -13,7 +13,14 @@ device (`ebc_local_map_angular`) for reset / step, like the reference does on ev
 (the reference computes and drops it there).  With use_grid_map = true it is the binary grid sub-map of env.py:630-708
 (`ebc_local_map_grid`: the window of scene.map around the robot, rotated like cv2.warpAffine does, thresholded).
 Rendering is out of scope.
+
+With the env INI's `[sim] orca_obstacles = true` (this project's key, off by default like the reference) humans avoid
+walls: every reset turns scene.obstacle_vertices -- generated or loaded from `load_scene_path` -- into RVO2 obstacle
+records on the device (`ebc_build_obstacles`, the same function BatchedEnv.reset_batch runs), and the lookahead's probe
+carries them too.
 """
+import dataclasses
+
 import numpy as np
 import torch
 
@@ -102,9 +109,9 @@ class EntityBasedCollisionAvoidance(object):
         pol = self.robot.policy
         A = len(pol.action_space) if getattr(pol, "action_space", None) else getattr(pol, "n_actions", 81)
         cfg = self._policy_config()
-        key = (H, S, R, A, cfg.robot_kinematics, cfg.with_agent_type, cfg.robot_visible)
+        key = (H, S, R, A, cfg.robot_kinematics, cfg.with_agent_type, cfg.robot_visible, cfg.orca_obstacles)
         if self.native is None or self._native_key != key:
-            self.native = BatchedSim(cfg, 1, H, S, R, A)
+            self.native = BatchedSim(cfg, 1, H, S, R, A, max_obst=64 if cfg.orca_obstacles else 0)
             self._native_key = key
             self._policy_bound = None
             self._probe = None
@@ -125,6 +132,10 @@ class EntityBasedCollisionAvoidance(object):
                                   np.array([R], np.int32), np.array([[rb.px, rb.py, rb.vx, rb.vy]], np.float32),
                                   np.array([[rb.gx, rb.gy, rb.v_pref, rb.radius]], np.float32),
                                   np.array([rb.theta], np.float32), np.array([self.global_time], np.float64))
+        if cfg.orca_obstacles:      # walls-aware humans: the scene's polygons -> RVO2 obstacle records, on the device
+            need = int(self.native.build_obstacles(*self._polygons())[0].item())
+            if need < 0:
+                raise abi.EbcError("the scene's obstacles need more than %d ORCA obstacle records" % self.native.Omax)
 
     def bind_policy(self, policy):
         """Register the policy's action table and value-network weights with the device (once per change)."""
@@ -176,7 +187,7 @@ class EntityBasedCollisionAvoidance(object):
         sim = n
         if ob is not None:
             if self._map_probe is None or self._map_probe.device != n.device:
-                self._map_probe = BatchedSim(n.cfg, 1, 1, 0, 0, 1, device=n.device)
+                self._map_probe = BatchedSim(dataclasses.replace(n.cfg, orca_obstacles=False), 1, 1, 0, 0, 1, device=n.device)
             sim = self._map_probe
             sim.rob_pv[0, 0], sim.rob_pv[0, 1] = float(ob.px), float(ob.py)
             sim.rob_gr[0, 3] = float(ob.radius)
@@ -195,7 +206,8 @@ class EntityBasedCollisionAvoidance(object):
         if ob is not None:
             # a one-episode probe that shares the scene's rectangle list
             if self._grid_probe is None or self._grid_probe.device != n.device or self._grid_probe.Rmax != n.Rmax:
-                self._grid_probe = BatchedSim(n.cfg, 1, 1, 0, n.Rmax, 1, device=n.device)
+                self._grid_probe = BatchedSim(dataclasses.replace(n.cfg, orca_obstacles=False), 1, 1, 0, n.Rmax, 1,
+                                              device=n.device)
             sim = self._grid_probe
             sim.rect.copy_(n.rect[:1])
             sim.rect_count.copy_(n.rect_count[:1])
@@ -298,10 +310,11 @@ class EntityBasedCollisionAvoidance(object):
         """Simulate one step without committing it; returns (next entity states, reward, done, info)."""
         n = self.native
         if self._probe is None:
-            self._probe = BatchedSim(n.cfg, 1, n.Hmax, n.Smax, n.Rmax, 1, device=n.device)
+            self._probe = BatchedSim(n.cfg, 1, n.Hmax, n.Smax, n.Rmax, 1, device=n.device, max_obst=n.Omax)
         p = self._probe
-        for name in ("hum_pv", "hum_gr", "hum_type", "hum_count", "stat", "stat_count", "rect", "rect_count",
-                     "rob_pv", "rob_gr", "rob_theta", "time"):
+        names = ("hum_pv", "hum_gr", "hum_type", "hum_count", "stat", "stat_count", "rect", "rect_count", "rob_pv",
+                 "rob_gr", "rob_theta", "time") + (("obst", "obst_count") if n.Omax else ())
+        for name in names:
             getattr(p, name).copy_(getattr(n, name))
         p.set_actions(np.array([self._action_pair(action)], dtype=np.float64))
         p.orca()

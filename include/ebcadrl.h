@@ -109,7 +109,9 @@ typedef struct ebc_config {
   float orca_time_horizon;           /* orca.py:66 (5) */
   /* ORCA obstacle half-planes (SURVEY 8f-4; spec: RVO2 computeNewVelocity obstacle section, caller
    * simulator/policy/orca_obstacles.py:83-152).  OFF by default = the reference's live behaviour: humans never see
-   * walls (orca.py adds no obstacle to its rvo2 sims). */
+   * walls (orca.py adds no obstacle to its rvo2 sims).  Turned on by this project's env INI key
+   * [sim] orca_obstacles = true; the records come from ebc_build_obstacles (the replayed scenes' polygons, on the
+   * device) or ebc_pack_obstacles (host). */
   int32_t orca_obstacles;            /* 1: humans (and the ORCA robot) avoid the episode's obstacle polygons */
   int32_t max_obst;                  /* Omax: obstacle-vertex slots per episode (0..64) */
   float orca_time_horizon_obst;      /* orca_obstacles.py:65 (5) */
@@ -126,7 +128,7 @@ typedef struct ebc_config {
 /* One RVO2 obstacle vertex (Obstacle.h: point_, unitDir_, nextObstacle_, prevObstacle_, isConvex_) plus this vertex's
  * place in RVO2's obstacle kd-tree (KdTree::buildObstacleTreeRecursive: one node per vertex, edges that straddle a
  * splitting line are split), from which every agent derives the tree's near-first visiting order for distance ties.
- * Produced on the host by ebc_pack_obstacles. */
+ * Produced by ebc_build_obstacles on the device or ebc_pack_obstacles on the host (the same function). */
 typedef struct ebc_obst_vertex {
   float px, py;         /* point_ */
   float ux, uy;         /* unitDir_ = normalize(next.point_ - point_) */
@@ -408,6 +410,15 @@ typedef struct ebc_replay_config {     /* one phase of SceneGenerator (scene_gen
 } ebc_replay_config;
 int ebc_replay_scenes(ebc_sim *sim, const ebc_replay_config *cfg, const uint32_t *seeds, const uint8_t *mask,
                       double *poly_xy, int32_t *poly_count, int32_t *need, void *stream);
+
+/* RVO2 addObstacle (each polygon of poly_xy, counter-clockwise as scene.obstacle_vertices stores them, narrowed to
+ * float like the rvo2 boundary) + processObstacles, per episode on the device, with the function ebc_pack_obstacles
+ * runs on the host.  For every episode e with mask[e] != 0 (mask NULL = all): writes state.obst[e] and obst_count[e];
+ * need[e] = the records the episode needs, or -1 when edge splitting exceeds cfg.max_obst (obst_count[e] = 0 then).
+ * Slots past obst_count[e] are left as they are.  EBC_ERR_INVALID unless cfg.orca_obstacles and max_obst >= 1.
+ * poly_xy [N*max_polys*4*2] f64, poly_count [N] i32: as ebc_replay_scenes writes them.  need [N] i32 (device). */
+int ebc_build_obstacles(ebc_sim *sim, const double *poly_xy, const int32_t *poly_count, int32_t max_polys,
+                        const uint8_t *mask, int32_t *need, void *stream);
 
 /* Angular local map of simulator/env.py:468-628 (SURVEY 8f-3): for every episode the distance to the closest
  * obstacle outline in each of `dim` angular sectors around the robot, in the robot's heading frame (angle 0 at
