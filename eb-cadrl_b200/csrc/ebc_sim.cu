@@ -1397,7 +1397,8 @@ angular_map_kernel(const ebc_config c, const ebc_state st, const ebc_angular_map
 // fixed-point terms (OpenCV's adelta / bdelta / X0 / Y0, 1/1024 units, cvRound = rint); (3) the window of scene.map is
 // rasterised from the episode's zero-cell rectangles into shared memory, one byte per cell, inside a one-cell frame
 // of ones (the constant border: a tap outside the window reads 1 without a bounds test); (4) every thread takes four
-// consecutive output cells: sample position to 1/32 pixel, four taps from shared memory, threshold, one 32-bit store.
+// consecutive output cells: sample position to 1/32 pixel, four taps from shared memory, threshold, one 32-bit store
+// (`packed`: the host's test that every episode's map starts on a 4-byte boundary; four byte stores otherwise).
 // The bilinear sum is taken in integers: OpenCV's float weights are (32 - fy)(32 - fx) / 1024 etc. (exact in
 // float), the taps are 0 or 1, so its float64 sum equals (integer sum) / 1024 exactly and "> 0.9" is "integer sum >=
 // 922" (0.9 * 1024 = 921.6) -- the oracle keeps OpenCV's float / double sequence, the tests demand equal cells.
@@ -1408,7 +1409,7 @@ struct GridMapShared {
 };
 
 __global__ void __launch_bounds__(256)
-grid_map_kernel(const ebc_config c, const ebc_state st, const int S, uint8_t *__restrict__ out) {
+grid_map_kernel(const ebc_config c, const ebc_state st, const int S, const bool packed, uint8_t *__restrict__ out) {
   extern __shared__ __align__(16) uint8_t gm_smem[];
   __shared__ GridMapShared sh;
   const int e = blockIdx.x, tid = threadIdx.x;
@@ -1470,7 +1471,6 @@ grid_map_kernel(const ebc_config c, const ebc_state st, const int S, uint8_t *__
     }
   }
   __syncthreads();
-  const bool packed = (cells & 3) == 0;
   for (int q = tid; 4 * q < cells; q += blockDim.x) {
     uint32_t word = 0;
     int y = (4 * q) / S, x = 4 * q - y * S;
@@ -1899,7 +1899,10 @@ int ebc_launch_grid_map(ebc_sim *s, const ebc_grid_map *map, uint8_t *out, cudaS
     grid_map_bits_kernel<<<s->cfg.n_episodes, 256, 0, stream>>>(s->cfg, s->st, S, magic, out);
     return ebc_check_launch(s, "grid_map_bits_kernel");
   }
-  grid_map_kernel<<<s->cfg.n_episodes, 256, smem, stream>>>(s->cfg, s->st, S, out);
+  // one 32-bit store per four cells only where every episode's map starts on a 4-byte boundary: S * S % 4 == 0 and
+  // an aligned `out` (the C API takes any uint8_t *, e.g. a view at an odd offset); byte stores otherwise
+  const bool packed = (S * S) % 4 == 0 && (uintptr_t)out % 4 == 0;
+  grid_map_kernel<<<s->cfg.n_episodes, 256, smem, stream>>>(s->cfg, s->st, S, packed, out);
   return ebc_check_launch(s, "grid_map_kernel");
 }
 

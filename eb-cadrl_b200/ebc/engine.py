@@ -356,7 +356,8 @@ class BatchedSim(object):
         poly_count = z(self.N, dtype=torch.int32) if poly_count is None else poly_count
         need = z(self.N, 5, dtype=torch.int32) if need is None else need
         assert tuple(poly_xy.shape) == (self.N, max(P, 1), 4, 2) and poly_xy.dtype == torch.float64 and poly_xy.is_contiguous()
-        assert tuple(need.shape) == (self.N, 5) and need.dtype == torch.int32 and poly_count.dtype == torch.int32
+        assert tuple(need.shape) == (self.N, 5) and need.dtype == torch.int32 and need.is_contiguous()
+        assert tuple(poly_count.shape) == (self.N,) and poly_count.dtype == torch.int32 and poly_count.is_contiguous()
         self.be.call("replay_scenes", self.h, ctypes.byref(config), _ptr(seeds), _ptr(mask), _ptr(poly_xy), _ptr(poly_count),
                      _ptr(need), stream=self._stream())
         return poly_xy, poly_count, need
@@ -369,7 +370,7 @@ class BatchedSim(object):
         edge splitting overflows Omax (obst_count is then 0); 0 for masked-off episodes."""
         assert poly_xy.dtype == torch.float64 and poly_xy.dim() == 4 and tuple(poly_xy.shape[2:]) == (4, 2)
         assert poly_xy.shape[0] == self.N and poly_xy.is_contiguous()
-        assert poly_count.dtype == torch.int32 and tuple(poly_count.shape) == (self.N,)
+        assert poly_count.dtype == torch.int32 and tuple(poly_count.shape) == (self.N,) and poly_count.is_contiguous()
         need = torch.zeros(self.N, dtype=torch.int32, device=self.device)
         self.be.call("build_obstacles", self.h, _ptr(poly_xy), _ptr(poly_count), poly_xy.shape[1], _ptr(mask), _ptr(need),
                      stream=self._stream())
@@ -390,11 +391,14 @@ class BatchedSim(object):
         """Angular local map of every episode (simulator/env.py:570-628, SURVEY 8f-3): `poly_xy` [N, Pmax, 4, 2]
         float64 = scene.obstacle_vertices, `poly_count` [N] int32; returns [N, dim] float64 on the device."""
         assert poly_xy.dtype == torch.float64 and poly_xy.dim() == 4 and tuple(poly_xy.shape[2:]) == (4, 2)
-        assert poly_xy.shape[0] == self.N and poly_count.dtype == torch.int32 and poly_count.shape[0] == self.N
+        assert poly_xy.shape[0] == self.N and poly_count.dtype == torch.int32 and tuple(poly_count.shape) == (self.N,)
+        assert poly_count.is_contiguous()
         if out is None:
             out = torch.empty(self.N, dim, dtype=torch.float64, device=self.device)
+        assert out.dtype == torch.float64 and tuple(out.shape) == (self.N, dim) and out.is_contiguous()
         m = abi.EbcAngularMap(max_range, min_angle, max_angle, dim, 1 if normalize else 0, poly_xy.shape[1], 0)
-        self.be.call("local_map_angular", self.h, ctypes.byref(m), _ptr(poly_xy.contiguous()), _ptr(poly_count),
+        poly_xy = poly_xy.contiguous()      # held until the call returns: a temporary copy would be freed before it
+        self.be.call("local_map_angular", self.h, ctypes.byref(m), _ptr(poly_xy), _ptr(poly_count),
                      _ptr(out), stream=self._stream())
         return out
 

@@ -456,7 +456,8 @@ typedef struct ebc_grid_map {
   int32_t size;          /* int(round(submap_size_m / map_resolution)), 1..192; must not exceed the map's cells */
   int32_t reserved;
 } ebc_grid_map;
-/* out [N*size*size] u8 (device). */
+/* out [N*size*size] u8 (device), contiguous, at any alignment: the kernel stores 4 cells per 32-bit word only where
+ * size*size % 4 == 0 and out is 4-byte aligned, and single bytes otherwise. */
 int ebc_local_map_grid(ebc_sim *sim, const ebc_grid_map *map, uint8_t *out, void *stream);
 
 /* ---- diagnostics (exported, but NOT part of the drop-in surface: nothing in the reference binds these;
